@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- fabric robot-steps/s of batched 3-Panda RF-CV rollouts (BASELINE.json's metric) on N B200s.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--batch B] [--horizon H]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--batch B] [--horizon H] [--dump-outputs DIR]
   N > 1:  python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
               bench.py --gpus N --steps K --warmup W
 
@@ -37,6 +37,14 @@ integrator update, avg-velocity accumulation).
             CPU arm is oracle O2 (closed-form C port, float64): ONE C call per step, goal estimate + rollout of every
             scenario inside one OpenMP loop on all host cores (thread count set explicitly, whatever OMP_NUM_THREADS
             the launcher exported), kind "port".
+  --dump-outputs DIR  (--impl ours only) what the last timed step of `value` computed, device layout (scenario axis
+            last) as float32 .npy: result (R+1,n) = avg_vel after the FP64 guard re-roll + deadlock flag, and the rollout's
+            avg_vel (R,n), x_ee (R,3,n), goal_est (3,n), risk (R,n); scenario_index.npy holds the n positions in the step's
+            batch that were written.  Written are the scenarios whose horizon the FP64 oracle finds calm (see calm(): the
+            few that blow up have NaN or overflowed outputs in every implementation), all of them up to 64 MB, beyond
+            that a fixed seeded sample; N > 1: one set per rank, suffix _rank<r>.  The timed batch itself is unchanged.
+            Inputs and selection depend only on the arguments, so two builds run with the same arguments can be
+            compared file for file.
 """
 from __future__ import annotations
 
@@ -73,7 +81,15 @@ def parse():
     ap.add_argument("--cpu-seconds", type=float, default=20.0, help="target duration of the CPU baseline sample")
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-f64", action="store_true", help="skip the FP64 sweep")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="--impl ours: write what the last timed step computed as DIR/<name>.npy (float32, at most 64 MB "
+                         "in all)")
+    a = ap.parse_args()
+    if a.steps < 1 or a.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours only")
+    return a
 
 
 def config_dict(a):
@@ -92,6 +108,16 @@ def _scenarios():
     """Scenario generator without touching the CUDA library (importing the package does not dlopen it)."""
     import multi_robot_fabrics_b200 as m
     return m.scenarios
+
+
+def calm(rec: np.ndarray, horizon: int) -> np.ndarray:
+    """(B,) mask of the scenarios (B,R,44) whose FP64 horizon (oracle O2) stays calm: avg_vel finite and below 2 for
+    every robot, the parity check's test.  The others blow up under explicit Euler near contact: velocities explode
+    within a few steps, a joint is thrown past its limit, the fabric metric stops being positive definite and every
+    implementation returns NaN or overflowed values (DESIGN.md section 2), so their outputs are not comparable."""
+    from oracle import o2
+    avg = o2.rollout_rfcv(o2.default_config(N_ROBOTS), rec.astype(np.float64), horizon, n_threads=o2.hw_threads())["avg_vel"]
+    return np.isfinite(avg).all(axis=1) & (avg.max(axis=1) < 2.0)
 
 
 def cpu_threads() -> int:
@@ -378,7 +404,27 @@ def _sweep(fab, torch, dist, dev, world, recs, works, H, steps, warmup, with_ris
     last = (warmup + steps - 1) % NBUF
     return dict(host_enqueue_ms=host_ms, total_ms=t0.elapsed_time(t1), kern_ms=[e0.elapsed_time(e1) for e0, e1 in kev],
                 avg=avg[last], flag=flag[last], result=results[steps - 1], last_set=(warmup + steps - 1) % len(recs),
+                x_ee=xee[last], goal_est=gest[last], risk=risk[last] if with_risk else None,
                 gathered=gathered, rollout_streams=len(roll))
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(path, arrays, keep, budget=DUMP_BYTES, suffix=""):
+    """--dump-outputs: arrays (name -> device tensor, scenario axis last) at the scenario positions `keep` (ascending)
+    as path/<name><suffix>.npy in float32, with scenario_index<suffix>.npy (float64) naming the positions written.
+    All of `keep` when it fits in `budget` bytes, otherwise the same seeded sample of it from every array, so that runs
+    with the same arguments write the same scenarios."""
+    import torch
+    per_scenario = 8 + sum(4 * t[..., 0].numel() for t in arrays.values())
+    n = min(len(keep), (budget - 128 * (len(arrays) + 1)) // per_scenario)  # 128: the header of a .npy file
+    idx = keep if n == len(keep) else np.sort(np.random.default_rng(0).choice(keep, size=n, replace=False))
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, f"scenario_index{suffix}.npy"), idx.astype(np.float64))
+    for name, t in arrays.items():
+        t = t.index_select(t.dim() - 1, torch.from_numpy(idx).to(t.device))
+        np.save(os.path.join(path, f"{name}{suffix}.npy"), t.float().cpu().numpy())
 
 
 def _isolated_kernel_ms(fab, torch, dev, recs, H, launches, with_risk=True):
@@ -445,6 +491,14 @@ def ours(a):
     sw = _sweep(fab, torch, dist, dev, world, recs, works, H, steps, warmup,
                 with_risk=os.environ.get("MRF_BENCH_NORISK", "0") != "1")
     clocks = sampler.stop()
+    if a.dump_outputs:
+        outs = {"result": sw["result"], "avg_vel": sw["avg"], "x_ee": sw["x_ee"], "goal_est": sw["goal_est"]}
+        if sw["risk"] is not None:
+            outs["risk"] = sw["risk"]
+        # the last step ran on a rolled record set: position i holds scenario (i - shift) % B of rec_h
+        pos = np.arange(B)
+        keep = pos[calm(rec_h, H)[(pos - (sw["last_set"] * B) // N_SETS) % B]]
+        dump_outputs(a.dump_outputs, outs, keep, DUMP_BYTES // world, suffix=f"_rank{rank}" if world > 1 else "")
     launches = (fab.handle.launches - launches0) * steps // (steps + warmup)
     total_ms = torch.tensor([sw["total_ms"]], dtype=torch.float64, device=dev)
     if world > 1:

@@ -175,30 +175,6 @@ def test_deadlock_restatement_point_mass_branch_matches_reference_golden():
     assert raised > 50
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/multi_robot_fabrics/others_planner/deadlock_prevention.py"),
-                    reason="reference tree only exists in the build container")
-def test_deadlock_restatement_matches_live_reference():
-    import importlib.util
-    spec = importlib.util.spec_from_file_location(
-        "ref_dlp", "/root/reference/multi_robot_fabrics/others_planner/deadlock_prevention.py")
-    mod = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(mod)
-    rng = np.random.default_rng(99)
-    for R in (2, 3):
-        ref, mine = mod.deadlockprevention([7] * R, R, 20), DeadlockOracle(R)
-        tdo_r = tdo_m = 1000
-        for t in range(200):
-            x = rng.uniform([0.3, -0.1, 1.0], [0.6, 0.1, 1.2], size=(R, 3))
-            goals = rng.uniform([0.2, -0.6, 0.8], [0.8, 0.6, 1.25], size=(R, 3))
-            w = rng.choice([2.0, 3.0], size=R)
-            avg = float(rng.uniform(0.0, 0.3))
-            st = list(rng.choice([0, 1, 1, 0, 2], size=R))
-            gr, wr, tdo_r = ref.deadlock_checking([v.copy() for v in x], [v.copy() for v in goals], list(w), t, tdo_r, avg, st)
-            gm, wm, tdo_m, _ = mine.step(x, goals, w, t, tdo_m, avg, st)
-            assert np.array_equal(np.array(gr, dtype=float), np.array(gm)) and tdo_r == tdo_m
-            assert [float(v) for v in wr] == [float(v) for v in wm]
-
-
 def test_sphere_offsets_and_sphere_kinematics(built):
     """Row 4 of the scope table: collision spheres with per-link offsets (create_simulation_manipulators.py:188-245,
     utils.py:87-119).  The package's offset table equals the oracle's restatement of the placement rule, and the
