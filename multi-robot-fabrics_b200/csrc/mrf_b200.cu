@@ -439,6 +439,15 @@ __global__ void __launch_bounds__(kTile* R, (R == 3 && sizeof(T) == 4) ? MRF_ROL
     }
     Chain<T> ch;
     const T vref = cfg.static_or_dyn ? T(1) : T(0), aref = cfg.static_or_dyn ? cfg.sref : T(0);
+    // shared robot-robot leaves (mrf_device.cuh, pair_leaves_eval): decided per scenario from its parameter blocks
+    constexpr bool kPair = kPairPath<T, R, UNIFORM>;
+    const bool pair_cfg = kPair && pair_leaves_cfg(cfg); // uniform over the grid: the extra barrier is not divergent
+    bool pair_on = false;
+    T* const pls = prm + P_N * NT;
+    if (pair_cfg) {
+        __syncthreads(); // every robot's parameter block is in shared memory
+        pair_on = pair_leaves_lane(prm, NT, lane);
+    }
     T acc = T(0);
     prm[P_RISK * NT + tid] = T(0); // running maximum of the stiffness indicator (shared memory: no register held)
     // k = -1: FK at the measured state only (end-effector position, RF-CV goal estimate); k >= 0: horizon steps.
@@ -489,7 +498,13 @@ __global__ void __launch_bounds__(kTile* R, (R == 3 && sizeof(T) == 4) ? MRF_ROL
         T act[kDof], stiff;
         if (UNIFORM) {
             SmemSrcUniform<T, R> src{kin, lane, r, vref, aref, cfg.r_obst};
-            fabric_action(cfg, r, q, qd, ch, kin, prm, NT, tid, src, act, &stiff);
+            PairLeaves<T> pl{T(0), pair_on};
+            if (pair_cfg) {
+                if (pair_on) pl.num = pair_leaves_eval(cfg, r, kin, prm, pls, NT, tid, lane);
+                __syncthreads(); // every robot's leaf slots are written
+                if (pair_on) pl.num += pls[2 * kPairSlots * NT + (r == 0 ? 2 : r - 1) * kTile + lane];
+            }
+            fabric_action(cfg, r, q, qd, ch, kin, prm, NT, tid, src, act, &stiff, kPair ? &pl : nullptr);
         } else {
             SmemSrc<T> src{cfg, kin, NT, lane, r, vref, aref, st_sph, AOS ? 0 : n_static, tid};
             fabric_action(cfg, r, q, qd, ch, kin, prm, NT, tid, src, act, &stiff);
@@ -1276,10 +1291,11 @@ static int rollout_dev(mrf_handle_t h, const T* rec, int N, T* avg_vel, T* x_ee,
     int rc = MRF_OK;
 #define MRF_LAUNCH_ROLLOUT_K(RR, UU, AA, SS)                                                                         \
     {                                                                                                                \
-        rc = set_smem(rollout_kernel<T, RR, UU, AA, SS>, smem);                                                      \
+        const size_t smem_k = smem + (kPairPath<T, RR, UU> ? sizeof(T) * (size_t)kPairRows * NT : 0);               \
+        rc = set_smem(rollout_kernel<T, RR, UU, AA, SS>, smem_k);                                                    \
         same_carveout(rollout_kernel<T, RR, UU, AA, SS>);                                                            \
         if (rc) return rc;                                                                                           \
-        rollout_kernel<T, RR, UU, AA, SS><<<(unsigned)grid, NT, smem, (cudaStream_t)stream>>>(                       \
+        rollout_kernel<T, RR, UU, AA, SS><<<(unsigned)grid, NT, smem_k, (cudaStream_t)stream>>>(                     \
             devcfg<T>(h), rec, N, avg_vel, x_ee, goal_est, qN, qdN, (long long)B, h->d_sync + 2 * sync_slot,        \
             (unsigned)h->zc_window, n_var, rec_tail, risk, ex);                                                      \
     }

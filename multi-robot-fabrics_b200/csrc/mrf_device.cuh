@@ -592,6 +592,179 @@ MRF_HD void sphere_leaf2(const V3<P2<T>>& p, const V3<P2<T>>& v, const V3<P2<T>>
     acc.b.x = pfma(d.x, gf, acc.b.x); acc.b.y = pfma(d.y, gf, acc.b.y); acc.b.z = pfma(d.z, gf, acc.b.z);
 }
 
+// ------------------------------------------------------------------------------------------------
+// Shared robot-robot leaves (FP32 throughput rollout of three robots with one sphere radius).  A leaf between point a
+// of robot i and point b of robot j is evaluated by both robots; swapping the roles gives d -> -d, w -> -w and leaves
+// n, g_s, 1/x, M_l, k = M_g g_s, u1, f_l and f_d unchanged when rho is the same on both sides.  The curvature term
+// becomes X_b = M_g (|w|^2 - d.c_b) + u1 rho' / n, and with vref = 1, aref = sigma (dynamic mode, jdot_sign ==
+// jdot_ref_sign) g_s f_q is the same on both sides: robot j's increments are A += k d d^T, b += g_s f_q d' with
+// d' = -d, and its energy term (d'.v_b) g_s ((sigma - 1) X_b + f_d) is one scalar.  So each leaf is evaluated once:
+// stage 1 (pair_leaves_eval) -- robot r against robot r+1, (k, g_s f_q) stored per leaf --, a CTA barrier, stage 2
+// (pair_leaves_rebuild inside fabric_action) -- every robot rebuilds its point accumulators from its own slots and from
+// robot r-1's.  -DMRF_NO_PAIR_LEAVES builds the kernels without it (every robot evaluates all its leaves).
+// ------------------------------------------------------------------------------------------------
+#ifdef MRF_NO_PAIR_LEAVES
+constexpr bool kPairLeaves = false;
+#else
+constexpr bool kPairLeaves = true;
+#endif
+constexpr int kTile = 32;                            // scenarios per CTA in the rollout kernel (one lane each)
+constexpr int kPairSlots = kEgo * (kPts / 2) * 2;    // per thread: (k, g_s f_q) of 5 ego points x 3 point pairs, as pairs
+constexpr int kPairRows = 2 * kPairSlots + 1;        // scalars per thread: the slots + the partner's energy sum
+template <typename T, int R, bool UNIFORM> constexpr bool kPairPath = kPairLeaves && UNIFORM && R == 3 && sizeof(T) == 4;
+
+// slot s of thread t holds a pair: scalars [(s * NT + t) * 2 + 0/1], one 64-bit access for FP32
+MRF_HD void pl_put(float* pl, int NT, int t, int s, P2<float> x) { reinterpret_cast<float2*>(pl)[s * NT + t] = x.v; }
+MRF_HD void pl_put(double* pl, int NT, int t, int s, P2<double> x) {
+    pl[(s * NT + t) * 2] = x.a;
+    pl[(s * NT + t) * 2 + 1] = x.b;
+}
+MRF_HD P2<float> pl_get(const float* pl, int NT, int t, int s) { return P2<float>{reinterpret_cast<const float2*>(pl)[s * NT + t]}; }
+MRF_HD P2<double> pl_get(const double* pl, int NT, int t, int s) { return pmk(pl[(s * NT + t) * 2], pl[(s * NT + t) * 2 + 1]); }
+template <typename T> MRF_HD T pl_half(const T* pl, int NT, int t, int s, int h) { return pl[(s * NT + t) * 2 + h]; }
+
+// The leaf slots follow the parameter blocks: prm + P_N * NT, kPairRows * NT scalars.
+template <typename T> struct PairLeaves {
+    T num;   // energy terms of the robot's leaves evaluated in stage 1, by itself and by robot r-1
+    bool on; // this lane's scenario takes the shared-leaf path (pair_leaves_lane)
+};
+
+// Configuration side of the condition: dynamic mode, sigma == aref, collision leaves on, three robots.
+template <typename T> MRF_HD bool pair_leaves_cfg(const DevCfg<T>& cfg) {
+    return cfg.n_robots == 3 && cfg.uniform_obst != 0 && cfg.has_coll != 0 && cfg.static_or_dyn != 0 && cfg.sigma == cfg.sref;
+}
+// Scenario side (per lane, so that a scenario's result never depends on its tile neighbours): every body radius of the
+// three robots is the same, so rho = r_obst + radius_body is one value for both sides of every leaf.
+template <typename T> MRF_HD bool pair_leaves_lane(const T* prm, int NT, int lane) {
+    const T r0 = prm[P_RB * NT + lane];
+    bool eq = true;
+    for (int j = 0; j < 3; ++j)
+#pragma unroll
+        for (int l = 0; l < 6; ++l) eq = eq && prm[(P_RB + l) * NT + j * kTile + lane] == r0;
+    return eq;
+}
+
+// Two leaves of the same ego point whose other sides are points of robot r+1 (dynamic mode, aref == sigma, rho passed
+// as in sphere_leaf2<T, true>): sphere_leaf2's algebra without the accumulation into A and b; returns k and g_s f_q,
+// accumulates the ego energy vector like sphere_leaf2 and the partner's energy term (d.v_b) g_e,b (negated by the caller).
+template <typename T>
+MRF_HD void sphere_leaf2_shared(const V3<P2<T>>& p, const V3<P2<T>>& v, const V3<P2<T>>& cc, const V3<P2<T>>& xo,
+                                const V3<P2<T>>& vo, const V3<P2<T>>& co, P2<T> nrho, P2<T> irho, P2<T> cM, T sigma,
+                                P2<T>& k, P2<T>& gf, V3<P2<T>>& nv, P2<T>& nvb) {
+    const P2<T> m1 = psplat(T(-1));
+    V3<P2<T>> d{pfma(xo.x, m1, p.x), pfma(xo.y, m1, p.y), pfma(xo.z, m1, p.z)};
+    V3<P2<T>> w{pfma(vo.x, m1, v.x), pfma(vo.y, m1, v.y), pfma(vo.z, m1, v.z)};
+    P2<T> n2 = pdot(d, d);
+    P2<T> in1 = prsqrt(n2);
+    P2<T> gs = pmul(in1, irho);
+    P2<T> ix = prcp(pfma(n2, gs, m1));
+    P2<T> nrin = pmul(in1, nrho);
+    P2<T> dw = pdot(d, w), da = pdot(d, co);
+    P2<T> ww = pdot(w, w);
+    P2<T> wc = pfma(d.z, cc.z, pfma(d.y, cc.y, pfma(d.x, cc.x, ww))); // |w|^2 + d.c_a
+    P2<T> wcb = pfma(da, m1, ww);                                      // |w|^2 + d'.c_b
+    P2<T> ix2 = pmul(ix, ix), ix4 = pmul(ix2, ix2);
+    P2<T> Ml = pmul(cM, ix4);
+    P2<T> Mg = pmul(Ml, gs);
+    k = pmul(Mg, gs);
+    P2<T> u1 = pmul(k, pmul(dw, dw));
+    P2<T> hh = pmul(ix4, psplat(T(-0.5)));
+    P2<T> fl = pmul(u1, hh);
+    P2<T> fd = pmul(u1, pfma(ix, psplat(T(2)), hh));
+    P2<T> X = pfma(u1, nrin, pmul(Mg, wc));
+    P2<T> Xb = pfma(u1, nrin, pmul(Mg, wcb));
+    P2<T> fq = pfma(X, psplat(sigma), pfma(pmul(Mg, da), psplat(-sigma), fl));
+    const P2<T> s1 = psplat(sigma - T(1));
+    P2<T> ge = pmul(gs, pfma(X, s1, fd));
+    nv.x = pfma(d.x, ge, nv.x); nv.y = pfma(d.y, ge, nv.y); nv.z = pfma(d.z, ge, nv.z);
+    P2<T> geb = pmul(gs, pfma(Xb, s1, fd));
+    nvb = pfma(pdot(d, vo), geb, nvb); // the constant point of robot r+1 has v = 0: no partner term
+    gf = pmul(gs, fq);
+}
+
+// Stage 1, thread (r, lane) of a pair lane: the 5 x 6 leaves of robot r's ego points against robot r+1's points (25
+// shared, 5 one-sided against r+1's constant link1==2 point) as sphere_leaf2 pairs; (k, g_s f_q) to the slots
+// (e * 3 + pp) * 2 + 0 / 1, the partner's energy sum to row 2 * kPairSlots.  Returns robot r's own energy terms.
+template <typename T>
+MRF_HD T pair_leaves_eval(const DevCfg<T>& cfg, int r, const T* kin, const T* prm, T* pl, int NT, int tid, int lane) {
+    const int t = (r == 2 ? 0 : r + 1) * kTile + lane;
+    const T rho = cfg.r_obst + prm[P_RB * NT + tid];
+    const P2<T> irho = psplat(Mth<T>::rcp(rho)), nrho = psplat(-rho);
+    T num = T(0);
+    P2<T> nvb = psplat(T(0));
+#pragma unroll 1
+    for (int e = 0; e < kEgo; ++e) {
+        const V3<T> p = kin_load(kin, NT, tid, e, 0), v = kin_load(kin, NT, tid, e, 3), cc = kin_load(kin, NT, tid, e, 6);
+        const V3<P2<T>> p2{psplat(p.x), psplat(p.y), psplat(p.z)}, v2{psplat(v.x), psplat(v.y), psplat(v.z)},
+            c2{psplat(cc.x), psplat(cc.y), psplat(cc.z)};
+        const T cw = T(0.02) * (e == 2 ? T(2) : T(1)); // link5 == link6
+        V3<P2<T>> nv{psplat(T(0)), psplat(T(0)), psplat(T(0))};
+#pragma unroll
+        for (int pp = 0; pp < kPts / 2; ++pp) {
+            P2<T> k, gf;
+            sphere_leaf2_shared(p2, v2, c2, kin_load_pair(kin, NT, t, pp, 0), kin_load_pair(kin, NT, t, pp, 3),
+                                kin_load_pair(kin, NT, t, pp, 6), nrho, irho,
+                                pmk(pp == 1 ? T(2) * cw : cw, pp == 2 ? T(2) * cw : cw), cfg.sigma, k, gf, nv, nvb);
+            pl_put(pl, NT, tid, (e * 3 + pp) * 2, k);
+            pl_put(pl, NT, tid, (e * 3 + pp) * 2 + 1, gf);
+        }
+        num = Mth<T>::fma(v.x, plo(nv.x) + phi(nv.x),
+                          Mth<T>::fma(v.y, plo(nv.y) + phi(nv.y), Mth<T>::fma(v.z, plo(nv.z) + phi(nv.z), num)));
+    }
+    pl[2 * kPairSlots * NT + tid] = -(plo(nvb) + phi(nvb));
+    return num;
+}
+
+// Stage 2, ego point e of thread (r, lane) of a pair lane, after the barrier: the one-sided leaf against robot r-1's
+// constant point (evaluated here), then the leaves e shares with robot r+1 (this thread's slots) and with robot r-1
+// (r-1's slots for its points 0..4 against point e) rebuilt from k and g_s f_q with d = p - x_o from the point table.
+template <typename T>
+MRF_HD void pair_leaves_rebuild(const DevCfg<T>& cfg, int r, const T* kin, const T* pl, int NT, int tid, int lane, int e,
+                                V3<T> p, V3<T> v, V3<T> cc, T rb, T we, PointAcc<T>& acc, T& num) {
+    const int tn = (r == 2 ? 0 : r + 1) * kTile + lane, tp = (r == 0 ? 2 : r - 1) * kTile + lane;
+    const V3<P2<T>> x2p = kin_load_pair(kin, NT, tp, 2, 0); // robot r-1's link8 | link1==2
+    const T rho = cfg.r_obst + rb;
+    const V3<T> z0 = mk(T(0), T(0), T(0));
+    sphere_leaf<T, true>(p, v, cc, mk(phi(x2p.x), phi(x2p.y), phi(x2p.z)), z0, z0, T(0), T(0), rho, T(2) * we, cfg.sigma,
+                         acc, num, Mth<T>::rcp(rho));
+    const int pe = e >> 1, he = e & 1; // point e in the point-pair numbering of the slots
+    {
+        const V3<T> d = p - mk(plo(x2p.x), plo(x2p.y), plo(x2p.z));
+        const int s = (4 * 3 + pe) * 2;
+        const T k = pl_half(pl, NT, tp, s, he), gf = pl_half(pl, NT, tp, s + 1, he);
+        const V3<T> Md = d * k;
+        acc.A.xx = Mth<T>::fma(Md.x, d.x, acc.A.xx); acc.A.xy = Mth<T>::fma(Md.x, d.y, acc.A.xy);
+        acc.A.xz = Mth<T>::fma(Md.x, d.z, acc.A.xz); acc.A.yy = Mth<T>::fma(Md.y, d.y, acc.A.yy);
+        acc.A.yz = Mth<T>::fma(Md.y, d.z, acc.A.yz); acc.A.zz = Mth<T>::fma(Md.z, d.z, acc.A.zz);
+        acc.b.x = Mth<T>::fma(d.x, gf, acc.b.x); acc.b.y = Mth<T>::fma(d.y, gf, acc.b.y); acc.b.z = Mth<T>::fma(d.z, gf, acc.b.z);
+    }
+    // the scalar sums seed the lo halves of the pair accumulators (as in fabric_action's sphere_leaf2 path)
+    const P2<T> m1 = psplat(T(-1));
+    Sym3<P2<T>> A{pmk(acc.A.xx, T(0)), pmk(acc.A.xy, T(0)), pmk(acc.A.xz, T(0)), pmk(acc.A.yy, T(0)), pmk(acc.A.yz, T(0)),
+                  pmk(acc.A.zz, T(0))};
+    V3<P2<T>> b{pmk(acc.b.x, T(0)), pmk(acc.b.y, T(0)), pmk(acc.b.z, T(0))};
+    const V3<P2<T>> p2{psplat(p.x), psplat(p.y), psplat(p.z)};
+    auto add = [&](const V3<P2<T>>& xo, P2<T> k, P2<T> gf) {
+        const V3<P2<T>> d{pfma(xo.x, m1, p2.x), pfma(xo.y, m1, p2.y), pfma(xo.z, m1, p2.z)};
+        const V3<P2<T>> Md{pmul(d.x, k), pmul(d.y, k), pmul(d.z, k)};
+        A.xx = pfma(Md.x, d.x, A.xx); A.xy = pfma(Md.x, d.y, A.xy); A.xz = pfma(Md.x, d.z, A.xz);
+        A.yy = pfma(Md.y, d.y, A.yy); A.yz = pfma(Md.y, d.z, A.yz); A.zz = pfma(Md.z, d.z, A.zz);
+        b.x = pfma(d.x, gf, b.x); b.y = pfma(d.y, gf, b.y); b.z = pfma(d.z, gf, b.z);
+    };
+#pragma unroll
+    for (int pp = 0; pp < kPts / 2; ++pp)
+        add(kin_load_pair(kin, NT, tn, pp, 0), pl_get(pl, NT, tid, (e * 3 + pp) * 2), pl_get(pl, NT, tid, (e * 3 + pp) * 2 + 1));
+#pragma unroll
+    for (int pp = 0; pp < 2; ++pp) {
+        const int s0 = ((2 * pp) * 3 + pe) * 2, s1 = ((2 * pp + 1) * 3 + pe) * 2;
+        add(kin_load_pair(kin, NT, tp, pp, 0), pmk(pl_half(pl, NT, tp, s0, he), pl_half(pl, NT, tp, s1, he)),
+            pmk(pl_half(pl, NT, tp, s0 + 1, he), pl_half(pl, NT, tp, s1 + 1, he)));
+    }
+    acc.A.xx = plo(A.xx) + phi(A.xx); acc.A.xy = plo(A.xy) + phi(A.xy); acc.A.xz = plo(A.xz) + phi(A.xz);
+    acc.A.yy = plo(A.yy) + phi(A.yy); acc.A.yz = plo(A.yz) + phi(A.yz); acc.A.zz = plo(A.zz) + phi(A.zz);
+    acc.b.x = plo(b.x) + phi(b.x); acc.b.y = plo(b.y) + phi(b.y); acc.b.z = plo(b.z) + phi(b.z);
+}
+
 // Plane leaf (geometry_plane_constraint "10*(1/(1+exp(-10x))-1) xdot^2", example_pandas_Jointspace.py:87;
 // finsler "0.1/x^2 s xdot^2", fabrics default)
 template <typename T>
@@ -792,8 +965,11 @@ template <typename T> MRF_HD void attractor_scalars(T n, T w, T& dpsi, T& m2) {
 // ------------------------------------------------------------------------------------------------
 template <typename T, typename Src>
 MRF_HD void fabric_action(const DevCfg<T>& cfg, int r, const T* q, const T* qd, const Chain<T>& ch, const T* kin,
-                          const T* prm, int NT, int tid, const Src& src, T* act, T* stiff = nullptr) {
+                          const T* prm, int NT, int tid, const Src& src, T* act, T* stiff = nullptr,
+                          const PairLeaves<T>* pair = nullptr) {
     const T sigma = cfg.sigma;
+    // shared robot-robot leaves (pair_leaves_eval has run for this step): the sphere leaves come from the slots
+    const bool pair_on = kPairLeaves && Src::kUniformRadius && pair != nullptr && pair->on;
     // stiffness indicator of this evaluation: sum over the ego points of trace(A_e) = sum over the collision leaves of
     // M_l |grad x|^2 (sphere leaf: 0.02 w / (x^4 rho^2), plane leaf: 0.2 s / x^2).  Near contact it explodes like 1/x^4;
     // the FP32 rollouts use its maximum over the horizon to decide which scenarios are re-rolled in FP64 (mrf_rfcv_post).
@@ -808,7 +984,7 @@ MRF_HD void fabric_action(const DevCfg<T>& cfg, int r, const T* q, const T* qd, 
     }
     G.m7 = T(0.2);
     G.f[6] = T(0);
-    T num = T(0); // qdot . (f_g - f_e,g)
+    T num = pair_on ? pair->num : T(0); // qdot . (f_g - f_e,g)
 
     // ---- joint-limit leaves (limit_geometry "-0.1/x xdot^2", limit_finsler "0.1/x s xdot^2") ----
     // lower and upper leaf of a joint as one pair (x = q - lo | hi - q, xdot = qd | -qd):
@@ -982,7 +1158,7 @@ MRF_HD void fabric_action(const DevCfg<T>& cfg, int r, const T* q, const T* qd, 
             const T rb0 = rb;
             for (int pass = 0; pass < passes; ++pass) {
                 if (pass == 1) rb = prm[(P_RB + rb_first + 1) * NT + tid];
-                if (!kPackedSpheres && !kObstMajor && !kObstMajorD) {
+                if (!kPackedSpheres && !kObstMajor && !kObstMajorD && !pair_on) {
                     // FP64: no packed instructions exist and pairing doubles the live registers -> one leaf at a time
                     if constexpr (Src::kUniformRadius) {
                         const T rho = src.ro + rb, irho = Mth<T>::rcp(rho); // one rho for every leaf of this ego point
@@ -1004,7 +1180,9 @@ MRF_HD void fabric_action(const DevCfg<T>& cfg, int r, const T* q, const T* qd, 
                     });
                 plane_leaf(p, v, cc, nh, dn, rb, we, sigma, acc, num);
             }
-            if (kPackedSpheres) {
+            if (pair_on) {
+                pair_leaves_rebuild(cfg, r, kin, prm + P_N * NT, NT, tid, tid % kTile, e, p, v, cc, rb0, we, acc, num);
+            } else if (kPackedSpheres) {
                 // ... then the FP32 sphere leaves two at a time with packed FP32x2 instructions (sm_100a FFMA2 / FMUL2); the
                 // scalar sums seed the lo halves of the pair accumulators, so folding the pairs is one addition per entry
                 PointAcc2<T> acc2;
@@ -1169,8 +1347,6 @@ MRF_HD void fabric_action(const DevCfg<T>& cfg, int r, const T* q, const T* qd, 
         act[i] = cfg.mode == 1 ? qd[i] + cfg.dt * qdd : qdd;
     }
 }
-
-constexpr int kTile = 32; // scenarios per CTA in the rollout kernel (one lane each)
 
 // ------------------------------------------------------------------------------------------------
 // obstacle sources for fabric_action
