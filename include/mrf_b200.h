@@ -15,6 +15,9 @@
  *                         end-effector FK of :236-238,328-329 fused in)
  *   mrf_rollout_cart_*    FabricsRollouts.symbolic_forward_fabrics + rollouts_numerical + get_velocity_rollouts
  *                         multi_robot_fabrics/fabrics_planner/forward_planner_Cartesian.py:347-489,538-563
+ *   mrf_rollout_cart_all_* the same for every robot of the handle in one launch: the per-robot FabricsRollouts calls of
+ *                         examples/example_pandas_cartesian.py:361-418 (one rollouts_numerical per robot, each against
+ *                         its own obstacle list)
  *   mrf_deadlock_*        deadlockprevention.deadlock_checking
  *                         multi_robot_fabrics/others_planner/deadlock_prevention.py:50-118
  *   mrf_kinematics_*      UtilsKinematics.necessary_kinematics fk/jac/jac_dot functions
@@ -27,7 +30,9 @@
  *   mrf_point_action_*    point-mass planner compute_action (examples/example_pointmasses_static.py:102-129,191-199)
  *   mrf_fsm_*             StateMachine.get_state_machine_panda + gripper action
  *                         multi_robot_fabrics/others_planner/state_machine.py:70-84,133-214
- *   mrf_episode_step_*    one iteration of the control loop examples/example_pandas_Jointspace.py:280-458
+ *   mrf_episode_step_*    one iteration of the control loop examples/example_pandas_Jointspace.py:280-458 (coupled
+ *                         joint-space rollouts) or examples/example_pandas_cartesian.py:295-462 (decoupled Cartesian rollouts,
+ *                         MrfEpisode.rollout_model = 1)
  *   mrf_rollout_host_submit_* / _wait   get_velocity_rollouts for a stream of independent batches (sweeps)
  *
  * Conventions
@@ -144,6 +149,15 @@ int mrf_rollout_cart_dev_f64(mrf_handle_t h, int robot, const double* rec, int S
                              double* avg_vel, double* qN, double* qdN, int64_t B, void* stream);
 int mrf_rollout_cart_dev_f32(mrf_handle_t h, int robot, const float* rec, int S, const float* obst, int N,
                              float* avg_vel, float* qN, float* qdN, int64_t B, void* stream);
+/* Cartesian (decoupled) rollouts of EVERY robot of the handle in one launch, each robot against its own obstacle list
+ * (the per-robot FabricsRollouts.rollouts_numerical / get_velocity_rollouts calls of
+ * examples/example_pandas_cartesian.py:361-418; forward_planner_Cartesian.py:421-458 per robot).  Layouts of
+ * mrf_action_dev_*:  rec [MRF_REC][R][B]  obst [S][MRF_OBST][R][B] (xddot ignored)  avg_vel [R][B]
+ * qN, qdN [R][N][MRF_DOF][B] (nullable).  Robot r's results equal those of mrf_rollout_cart_dev_*(robot = r) on its slices. */
+int mrf_rollout_cart_all_dev_f64(mrf_handle_t h, const double* rec, int S, const double* obst, int N, double* avg_vel,
+                                 double* qN, double* qdN, int64_t B, void* stream);
+int mrf_rollout_cart_all_dev_f32(mrf_handle_t h, const float* rec, int S, const float* obst, int N, float* avg_vel,
+                                 float* qN, float* qdN, int64_t B, void* stream);
 
 /* Link kinematics of the 8 collision links: x, v = J qdot, a = jdot_ref_sign * d(J qdot)/dq qdot.
  *   q, qdot [MRF_DOF][R][B];  x, v, a [MRF_NLINKS][3][R][B] (nullable) */
@@ -339,14 +353,25 @@ int mrf_deadlock_host_f64(mrf_handle_t h, const double* x_ee, double* goals, dou
  *   link, link-origin velocities (:400-412) -> executed action with weight_goal_1 = w1_action (:417-445) -> clip (:453),
  *   integrate, metrics (first step at which the task is reached, minimum sphere clearance :461-470, deadlock steps).
  * Seven kernel launches on `stream`; capture it in a CUDA graph and replay.  All pointers are device pointers of the
- * entry's precision (T) unless typed; b fastest. */
+ * entry's precision (T) unless typed; b fastest.
+ * rollout_model = 1 runs the loop body of examples/example_pandas_cartesian.py:295-462 instead
+ * (rollouts: forward_planner_Cartesian.py:421-458): clip ->
+ * hand FK and J qdot at the measured state (kin_scratch) -> RF-CV goal x_hand + estimate_horizon * J qdot of robot
+ * `estimate_robot` written into its goal rows before the rollouts (:355-357; any nonzero MrfConfig.estimate_goal takes
+ * this J qdot form here, 2 in MrfConfig terms) -> every robot's
+ * sphere list with true sphere velocities (mrf_obstacles_dev vel_mode 1, :343-352) -> mrf_rollout_cart_all_dev with
+ * weight_goal_1 = w1_rollout (20, :42) -> deadlock_checking on sum(avg_vel) / R (:405) -> the executed action as above
+ * (link-origin velocities, vel_mode 0).  The rollouts use the planner with collision links in every state. */
 typedef struct MrfEpisode {
     int32_t struct_size;        /* sizeof(MrfEpisode) */
     int32_t n_horizon;          /* rollout horizon (rollout_fabrics) */
     int32_t rollout_fabrics;    /* 0 = MRDF: no rollouts, no deadlock logic */
     int32_t resolve_deadlocks;
-    int32_t n_per_link;         /* collision spheres per link seen by the executed action */
-    int32_t reserved0;
+    int32_t n_per_link;         /* collision spheres per link seen by the executed action (and by the Cartesian rollouts) */
+    int32_t rollout_model;      /* read when rollout_fabrics = 1.  0: coupled joint-space rollouts (ForwardFabricsPlanner,
+                                   examples/example_pandas_Jointspace.py:352-376).  1: decoupled Cartesian rollouts
+                                   (FabricsRollouts, examples/example_pandas_cartesian.py:343-418): each robot rolled out
+                                   alone against the other robots' spheres moving at constant velocity; needs kin_scratch */
     double epsilon;             /* reach tolerance (0.05) */
     double w1_rollout, w1_action;   /* weight_goal_1: 10 in the rollouts (:43,364), 20 in the executed action (:427) */
     double clearance_radius_sum;    /* subtracted from sphere-centre distances (0.16) */
@@ -361,7 +386,7 @@ typedef struct MrfEpisode {
     void* obst;                 /* T [8 n (R-1)][MRF_OBST][R][B] */
     void* spheres_x;            /* T [8 n][3][R][B] */
     void* action;               /* T [MRF_DOF][R][B] */
-    void* kin_scratch;          /* T [3][8][3][R][B] (MRDF mode only) */
+    void* kin_scratch;          /* T [3][8][3][R][B] (MRDF mode, pick-and-place, rollout_model = 1) */
     const int32_t* sm_state;    /* [R][B] state-machine codes (resolve_deadlocks) */
     int32_t* time_step;         /* [B] in/out, incremented */
     int32_t* time_deadlock_out; /* [B] in/out */

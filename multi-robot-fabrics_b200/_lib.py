@@ -43,7 +43,7 @@ class MrfEpisode(C.Structure):
     """include/mrf_b200.h: state of mrf_episode_step_dev_* (device pointers as integers)."""
     _fields_ = [
         ("struct_size", C.c_int32), ("n_horizon", C.c_int32), ("rollout_fabrics", C.c_int32),
-        ("resolve_deadlocks", C.c_int32), ("n_per_link", C.c_int32), ("reserved0", C.c_int32),
+        ("resolve_deadlocks", C.c_int32), ("n_per_link", C.c_int32), ("rollout_model", C.c_int32),
         ("epsilon", C.c_double), ("w1_rollout", C.c_double), ("w1_action", C.c_double),
         ("clearance_radius_sum", C.c_double), ("vel_limit", C.c_double * DOF),
         ("offsets", C.c_void_p), ("rec", C.c_void_p), ("goal0", C.c_void_p), ("w0", C.c_void_p), ("avg_vel", C.c_void_p),
@@ -64,7 +64,8 @@ _F = {"f32": (C.c_float, np.float32), "f64": (C.c_double, np.float64)}
 EXPORTS = [
     "mrf_version", "mrf_last_error", "mrf_config_default", "mrf_create", "mrf_destroy", "mrf_device_count",
     "mrf_action_dev_f64", "mrf_action_dev_f32", "mrf_rollout_dev_f64", "mrf_rollout_dev_f32",
-    "mrf_rollout_cart_dev_f64", "mrf_rollout_cart_dev_f32", "mrf_kinematics_dev_f64", "mrf_kinematics_dev_f32",
+    "mrf_rollout_cart_dev_f64", "mrf_rollout_cart_dev_f32", "mrf_rollout_cart_all_dev_f64", "mrf_rollout_cart_all_dev_f32",
+    "mrf_kinematics_dev_f64", "mrf_kinematics_dev_f32",
     "mrf_deadlock_dev_f64", "mrf_deadlock_dev_f32", "mrf_deadlock_rec_dev_f64", "mrf_deadlock_rec_dev_f32", "mrf_fsm_dev_f64", "mrf_fsm_dev_f32", "mrf_obstacles_dev_f64", "mrf_obstacles_dev_f32", "mrf_point_action_dev_f64", "mrf_point_action_dev_f32",
     "mrf_point_action_host_f64", "mrf_action_host_f64", "mrf_action_host_f32",
     "mrf_rollout_host_f64", "mrf_rollout_host_f32", "mrf_rollout_cart_host_f64", "mrf_rollout_cart_host_f32",
@@ -101,6 +102,7 @@ def lib():
         getattr(L, f"mrf_action_dev_{p}").argtypes = [vp, i32, i32, vp, i32, vp, vp, i64, vp]
         getattr(L, f"mrf_rollout_dev_{p}").argtypes = [vp, vp, i32, vp, vp, vp, vp, vp, i64, vp]
         getattr(L, f"mrf_rollout_cart_dev_{p}").argtypes = [vp, i32, vp, i32, vp, i32, vp, vp, vp, i64, vp]
+        getattr(L, f"mrf_rollout_cart_all_dev_{p}").argtypes = [vp, vp, i32, vp, i32, vp, vp, vp, i64, vp]
         getattr(L, f"mrf_kinematics_dev_{p}").argtypes = [vp, vp, vp, vp, vp, vp, i64, vp]
         getattr(L, f"mrf_deadlock_dev_{p}").argtypes = [vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, i64, vp]
         getattr(L, f"mrf_deadlock_rec_dev_{p}").argtypes = [vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, i64, vp]

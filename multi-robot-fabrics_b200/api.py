@@ -333,6 +333,29 @@ class Fabrics:
                  self._tp(qdN), B, self._stream()), "mrf_rollout_cart_dev")
         return avg_vel
 
+    def rollout_cart_all_dev(self, rec, obst, N: int, avg_vel=None, qN=None, qdN=None):
+        """Cartesian rollouts of every robot in one launch (mrf_rollout_cart_all_dev): rec (44,R,B), obst (S,10,R,B) or
+        None -> avg_vel (R,B); qN, qdN (R,N,7,B) optional.  Robot r's results equal rollout_cart_dev(r, ...) on its slices."""
+        import torch
+        p = self._prec(rec)
+        R = self.n_robots
+        if rec.dim() != 3:
+            raise MrfError(f"rec must be a contiguous (44,{R},B) tensor")
+        B = rec.shape[-1]
+        dt, dev = rec.dtype, rec.device
+        _chk("rec", rec, (REC, R, B), optional=False)
+        S = 0 if obst is None else obst.shape[0]
+        _chk("obst", obst, (S, OBST, R, B), dt, dev)
+        if avg_vel is None:
+            avg_vel = torch.empty((R, B), dtype=dt, device=dev)
+        _chk("avg_vel", avg_vel, (R, B), dt, dev)
+        _chk("qN", qN, (R, N, DOF, B), dt, dev)
+        _chk("qdN", qdN, (R, N, DOF, B), dt, dev)
+        fn = getattr(lib(), f"mrf_rollout_cart_all_dev_{p}")
+        check(fn(self.handle.ptr, self._tp(rec), S, self._tp(obst), N, self._tp(avg_vel), self._tp(qN), self._tp(qdN), B,
+                 self._stream()), "mrf_rollout_cart_all_dev")
+        return avg_vel
+
     def kinematics_dev(self, q, qdot, x=None, v=None, a=None):
         import torch
         p = self._prec(q)

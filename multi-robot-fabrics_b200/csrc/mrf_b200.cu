@@ -597,8 +597,10 @@ __global__ void __launch_bounds__(kActThreads, sizeof(T) == 4 ? MRF_ACTION_MINBL
             for (int i = 0; i < kDof; ++i) out[(long long)i * stride + idx] = act[i];
         }
     } else {
-        // forward_planner_Cartesian.py:421-458: evaluate, then step robot and obstacles
+        // forward_planner_Cartesian.py:421-458: evaluate, then step robot and obstacles.  Outputs per robot of the call:
+        // avg_vel [n_rob][B], qN / qdN [n_rob][N][7][B] (n_rob = 1: the single-robot layouts [B], [N][7][B])
         T acc = T(0);
+        const long long tb = (long long)rl * N * kDof * B + b; // column of this thread in qN / qdN
         for (int k = 0; k < N; ++k) {
             T act[kDof];
             src.tk = T(k) * cfg.dt;
@@ -618,12 +620,12 @@ __global__ void __launch_bounds__(kActThreads, sizeof(T) == 4 ? MRF_ACTION_MINBL
             if (live) {
 #pragma unroll
                 for (int i = 0; i < kDof; ++i) {
-                    if (qN != nullptr) qN[((long long)k * kDof + i) * B + b] = q[i];
-                    if (qdN != nullptr) qdN[((long long)k * kDof + i) * B + b] = qd[i];
+                    if (qN != nullptr) qN[((long long)k * kDof + i) * B + tb] = q[i];
+                    if (qdN != nullptr) qdN[((long long)k * kDof + i) * B + tb] = qd[i];
                 }
             }
         }
-        if (out != nullptr && live) out[b] = acc / (T(N) * T(kDof));
+        if (out != nullptr && live) out[src.off] = acc / (T(N) * T(kDof)); // src.off == idx = rl * B + b
     }
 }
 
@@ -1450,6 +1452,16 @@ extern "C" int mrf_rollout_cart_dev_f64(mrf_handle_t h, int robot, const double*
 extern "C" int mrf_rollout_cart_dev_f32(mrf_handle_t h, int robot, const float* rec, int S, const float* obst, int N,
                                         float* avg_vel, float* qN, float* qdN, int64_t B, void* stream) {
     return action_dev<float, true>(h, robot, 1, rec, S, obst, N, avg_vel, qN, qdN, B, stream);
+}
+extern "C" int mrf_rollout_cart_all_dev_f64(mrf_handle_t h, const double* rec, int S, const double* obst, int N,
+                                            double* avg_vel, double* qN, double* qdN, int64_t B, void* stream) {
+    if (!h) return fail(MRF_EINVAL, "mrf_rollout_cart_all: null handle");
+    return action_dev<double, true>(h, 0, h->cfg.n_robots, rec, S, obst, N, avg_vel, qN, qdN, B, stream);
+}
+extern "C" int mrf_rollout_cart_all_dev_f32(mrf_handle_t h, const float* rec, int S, const float* obst, int N,
+                                            float* avg_vel, float* qN, float* qdN, int64_t B, void* stream) {
+    if (!h) return fail(MRF_EINVAL, "mrf_rollout_cart_all: null handle");
+    return action_dev<float, true>(h, 0, h->cfg.n_robots, rec, S, obst, N, avg_vel, qN, qdN, B, stream);
 }
 extern "C" int mrf_kinematics_dev_f64(mrf_handle_t h, const double* q, const double* qdot, double* x, double* v,
                                       double* a, int64_t B, void* stream) {
@@ -2441,10 +2453,14 @@ extern "C" int mrf_fsm_dev_f32(mrf_handle_t h, const int32_t* nr_blocks, const f
 struct EpLimits {
     double v[MRF_DOF];
 };
-// :288 velocity clip of the measured state; goals / weights of this step start from the task's own (:352-368)
+// :288 velocity clip of the measured state; goals / weights of this step start from the task's own (:352-368).
+// goal0 == nullptr: the clip only.  kin != nullptr (decoupled Cartesian rollouts): kin_scratch [3][8][3][R][B] of the
+// clipped state; robot est_robot's goal is the RF-CV estimate x_hand + est_h * J qdot when `estimate` is set
+// (example_pandas_cartesian.py:355-357), and goal_est [3][B] receives the goal that robot's rollout uses.
 template <typename T>
 __global__ void episode_pre_kernel(T* __restrict__ rec, const T* __restrict__ goal0, const T* __restrict__ w0, EpLimits lim,
-                                   T w1, int R, long long B) {
+                                   T w1, int R, long long B, const T* __restrict__ kin = nullptr, int est_robot = -1,
+                                   int estimate = 0, T est_h = T(0), T* __restrict__ goal_est = nullptr) {
     const long long RB = (long long)R * B, idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (idx >= RB) return;
     const int r = (int)(idx / B);
@@ -2455,8 +2471,20 @@ __global__ void episode_pre_kernel(T* __restrict__ rec, const T* __restrict__ go
         const T l = (T)lim.v[i], v = *p;
         *p = v < -l ? -l : (v > l ? l : v); // NaN stays NaN, like np.clip
     }
+    if (goal0 == nullptr) return;
+    const bool est_here = kin != nullptr && r == est_robot;
 #pragma unroll
-    for (int c = 0; c < 3; ++c) rec[(MRF_G0 + c) * RB + idx] = goal0[((long long)r * 3 + c) * B + b];
+    for (int c = 0; c < 3; ++c) {
+        T g = goal0[((long long)r * 3 + c) * B + b];
+        if (est_here) {
+            if (estimate) {
+                const T* hand = kin + (long long)(MRF_NLINKS - 1) * 3 * RB; // x of link 8; its v rows follow 8 * 3 rows on
+                g = hand[c * RB + idx] + hand[(long long)MRF_NLINKS * 3 * RB + c * RB + idx] * est_h;
+            }
+            if (goal_est != nullptr) goal_est[(long long)c * B + b] = g;
+        }
+        rec[(MRF_G0 + c) * RB + idx] = g;
+    }
     rec[MRF_W0 * RB + idx] = w0[idx];
     rec[MRF_W1 * RB + idx] = w1;
 }
@@ -2474,8 +2502,9 @@ __global__ void episode_mid_kernel(T* __restrict__ rec, const T* __restrict__ go
         for (int c = 0; c < 3; ++c) rec[(MRF_G0 + c) * RB + idx] = goal_est[(long long)c * B + b];
     }
 }
-// pick-and-place task (:289-303): hand position at the measured state for the state machine, and the block each robot
-// goes for next -- block number nr_blocks_success of its own stack, grasp height 0.1 above the block (:302-303)
+// hand position at the measured state (for the state machine and, with decoupled Cartesian rollouts, the deadlock
+// heuristic) and, in the pick-and-place task (:289-303, blocks != nullptr), the block each robot goes for next -- block
+// number nr_blocks_success of its own stack, grasp height 0.1 above the block (:302-303)
 template <typename T>
 __global__ void episode_blocks_kernel(const T* __restrict__ hand, T* __restrict__ x_ee, const T* __restrict__ blocks, int n_blocks,
                                       const int32_t* __restrict__ st, T* __restrict__ goal_block, int R, long long B) {
@@ -2483,7 +2512,7 @@ __global__ void episode_blocks_kernel(const T* __restrict__ hand, T* __restrict_
     if (idx >= RB) return;
     const int r = (int)(idx / B);
     const long long b = idx - (long long)r * B;
-    const int n_ok = st[1 * RB + idx];
+    const int n_ok = blocks != nullptr ? st[1 * RB + idx] : n_blocks;
 #pragma unroll
     for (int c = 0; c < 3; ++c) {
         x_ee[((long long)r * 3 + c) * B + b] = hand[((long long)c * R + r) * B + b];
@@ -2574,6 +2603,10 @@ template <typename T> static int episode_step_dev(mrf_handle_t h, const MrfEpiso
          !ep->deadlock_steps))
         return fail(MRF_EINVAL, "mrf_episode_step: deadlock resolution needs its state arrays");
     if (!ep->rollout_fabrics && !ep->kin_scratch) return fail(MRF_EINVAL, "mrf_episode_step: MRDF mode needs kin_scratch");
+    if (ep->rollout_fabrics && ep->rollout_model != 0 && ep->rollout_model != 1)
+        return fail(MRF_EINVAL, "mrf_episode_step: rollout_model must be 0 (coupled joint-space) or 1 (decoupled Cartesian)");
+    const bool cart = ep->rollout_fabrics && ep->rollout_model == 1;
+    if (cart && !ep->kin_scratch) return fail(MRF_EINVAL, "mrf_episode_step: Cartesian rollouts need kin_scratch");
     if (B <= 0) return fail(MRF_EINVAL, "mrf_episode_step: B must be positive");
     MRF_CUDA(cudaSetDevice(h->device));
     const int R = h->cfg.n_robots;
@@ -2586,6 +2619,11 @@ template <typename T> static int episode_step_dev(mrf_handle_t h, const MrfEpiso
     const bool est = h->cfg.estimate_goal != 0 && R > 1;
     const bool pnp = ep->pick_and_place != 0;
     const int32_t* sm_state = ep->sm_state;
+    if (cart) { // the velocity clip first: the kinematics below (hand, J qdot of the estimate) read the clipped state
+        episode_pre_kernel<T><<<g_rb, 256, 0, st>>>(rec, nullptr, nullptr, lim, T(0), R, (long long)B);
+        MRF_CUDA(cudaGetLastError());
+        h->launches += 1;
+    }
     if (pnp) {
         if (!ep->kin_scratch || !ep->blocks || !ep->q_grip || !ep->start_goal || !ep->goal_block || !ep->fsm_above || !ep->fsm_st ||
             !ep->grip_action || ep->n_blocks < 1)
@@ -2605,25 +2643,52 @@ template <typename T> static int episode_step_dev(mrf_handle_t h, const MrfEpiso
                          (T*)ep->goal0, (T*)ep->fsm_above, (T*)ep->w0, ep->fsm_st, (T*)ep->grip_action, B, stream);
         if (rc0) return rc0;
         sm_state = ep->fsm_st; // row 0 of [6][R][B] = state codes
+    } else if (cart) {
+        T* kx = (T*)ep->kin_scratch;
+        const size_t n = (size_t)MRF_NLINKS * 3 * RB;
+        int rc0 = kinematics_dev<T>(h, rec + MRF_Q * RB, rec + MRF_QD * RB, kx, kx + n, kx + 2 * n, B, stream);
+        if (rc0) return rc0;
+        episode_blocks_kernel<T><<<g_rb, 256, 0, st>>>(kx + (size_t)(MRF_NLINKS - 1) * 3 * RB, (T*)ep->x_ee, nullptr, 0,
+                                                       nullptr, nullptr, R, (long long)B);
+        MRF_CUDA(cudaGetLastError());
+        h->launches += 1;
     }
+    const int est_robot = (h->cfg.estimate_robot >= 0 && h->cfg.estimate_robot < R) ? h->cfg.estimate_robot : -1;
     episode_pre_kernel<T><<<g_rb, 256, 0, st>>>(rec, (const T*)ep->goal0, (const T*)ep->w0, lim,
-                                                (T)(ep->rollout_fabrics ? ep->w1_rollout : ep->w1_action), R, (long long)B);
+                                                (T)(ep->rollout_fabrics ? ep->w1_rollout : ep->w1_action), R, (long long)B,
+                                                cart ? (const T*)ep->kin_scratch : nullptr, est_robot, est ? 1 : 0,
+                                                (T)h->cfg.estimate_horizon, cart ? (T*)ep->goal_est : nullptr);
     MRF_CUDA(cudaGetLastError());
     h->launches += 1;
     int rc;
     const T* xee = (const T*)ep->x_ee;
     int link_major = 0;
+    const int S1 = MRF_NLINKS * ep->n_per_link;
     if (ep->rollout_fabrics) {
-        rc = rollout_dev<T>(h, rec, ep->n_horizon, (T*)ep->avg_vel, (T*)ep->x_ee, (T*)ep->goal_est, nullptr, nullptr, B, stream);
+        if (cart) {
+            // example_pandas_cartesian.py:343-352: each robot's rollout sees the other robots' spheres with their true
+            // velocities J_sphere qdot (compute_x_obsts_dyn_0, utils_apply_fk.py:3-33), moving at constant velocity over the
+            // horizon.  The executed action below keeps the joint-space loop's staging (link-origin velocities): the
+            // Cartesian example's action-side assembly is taken to be the same as the joint-space example's.
+            rc = obstacles_dev<T>(h, ep->n_per_link, ep->offsets, 1, rec + MRF_Q * RB, rec + MRF_QD * RB, (T*)ep->obst, nullptr,
+                                  nullptr, B, stream);
+            if (rc) return rc;
+            rc = action_dev<T, true>(h, 0, R, rec, S1 * (R - 1), (const T*)ep->obst, ep->n_horizon, (T*)ep->avg_vel, nullptr,
+                                     nullptr, B, stream);
+        } else {
+            rc = rollout_dev<T>(h, rec, ep->n_horizon, (T*)ep->avg_vel, (T*)ep->x_ee, (T*)ep->goal_est, nullptr, nullptr, B,
+                                stream);
+        }
         if (rc) return rc;
+        // Cartesian: the estimate already sits in the record's goal rows (episode_pre_kernel)
+        const T* gest = (est && !cart) ? (const T*)ep->goal_est : nullptr;
         if (ep->resolve_deadlocks && R >= 2) { // the heuristic is defined on robot pairs
-            rc = deadlock_rec_dev<T>(h, (const T*)ep->x_ee, rec, est ? (const T*)ep->goal_est : nullptr, (const T*)ep->avg_vel,
-                                     nullptr, sm_state, ep->time_step, ep->time_deadlock_out, ep->st_int, (T*)ep->st_goal,
-                                     ep->flag, B, stream);
+            rc = deadlock_rec_dev<T>(h, (const T*)ep->x_ee, rec, gest, (const T*)ep->avg_vel, nullptr, sm_state, ep->time_step,
+                                     ep->time_deadlock_out, ep->st_int, (T*)ep->st_goal, ep->flag, B, stream);
             if (rc) return rc;
         }
-        episode_mid_kernel<T><<<g_rb, 256, 0, st>>>(rec, (est && !ep->resolve_deadlocks) ? (const T*)ep->goal_est : nullptr,
-                                                    h->cfg.estimate_robot, (T)ep->w1_action, R, (long long)B);
+        episode_mid_kernel<T><<<g_rb, 256, 0, st>>>(rec, !ep->resolve_deadlocks ? gest : nullptr, h->cfg.estimate_robot,
+                                                    (T)ep->w1_action, R, (long long)B);
         MRF_CUDA(cudaGetLastError());
         h->launches += 1;
     } else if (!pnp) {
@@ -2634,7 +2699,6 @@ template <typename T> static int episode_step_dev(mrf_handle_t h, const MrfEpiso
         xee = kx + (size_t)(MRF_NLINKS - 1) * 3 * RB; // hand rows [3][R][B]
         link_major = 1;
     }
-    const int S1 = MRF_NLINKS * ep->n_per_link;
     rc = obstacles_dev<T>(h, ep->n_per_link, ep->offsets, 0, rec + MRF_Q * RB, rec + MRF_QD * RB, (T*)ep->obst, (T*)ep->spheres_x,
                           nullptr, B, stream);
     if (rc) return rc;

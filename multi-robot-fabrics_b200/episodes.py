@@ -15,30 +15,51 @@ device every step -- it sets goals / weight_goal_0, gates the deadlock logic, sw
 planner in state 2, holds the arm while gripping / releasing and drives the finger joints; blocks are kinematic (picked
 in order, never dropped); an episode succeeds when every robot has picked all its blocks (state 10).  One control step is ONE C-ABI call (mrf_episode_step_dev_*: seven kernel launches), captured in a CUDA
 graph and replayed; torch only owns the tensors.
+
+Two rollout models (`rollouts=`).  "jointspace" (default) is the loop above: coupled ForwardFabricsPlanner rollouts.
+"cartesian" is the loop of examples/example_pandas_cartesian.py:295-462 (decoupled FabricsRollouts, one per robot):
+  1. velocity clip; end-effector FK and J qdot at the measured state; RF-CV goal of robot 1 = x_ee + 0.2 * J qdot
+     (the true hand velocity, estimate_goal = 2), written into its goal before the rollouts      :343-357
+  2. other robots' collision spheres with their true sphere velocities (compute_x_obsts_dyn_0)   :343-352
+  3. each robot's Cartesian rollout against those spheres moving at constant velocity, weight_goal_1 = 20 in the
+     rollouts as in the action (:42); all robots in one launch                                  :361-418
+  4. deadlock_checking on sum(avg_vel) / R                                                      :405
+  5.-6. obstacle staging with link-origin velocities, executed action, integration: as in the joint-space loop
+     (the Cartesian example's action-side staging is taken to be the joint-space example's).
+The rollouts always use the planner with collision links (no grasp planner inside the horizon), as the coupled ones do.
 """
 from __future__ import annotations
 
 import numpy as np
 
-from ._lib import G0, Q, QD, W0, W1
+from ._lib import G0, Q, QD, W0, W1, MrfError
 from .api import Fabrics, to_soa
 
 VEL_LIMITS = [2.175, 2.175, 2.175, 2.175, 2.61, 2.61, 2.61]          # example_pandas_Jointspace.py:221
+ROLLOUT_MODELS = {"jointspace": 0, "cartesian": 1}                    # MrfEpisode.rollout_model
 
 
 class BatchedEpisodes:
     def __init__(self, rec: np.ndarray, n_horizon: int = 10, rollout_fabrics: bool = True, resolve_deadlocks: bool = True,
                  estimate_goal: bool = False, static_or_dyn: int = 1, n_obst_per_link: int = 1, device: int = 0,
-                 dtype: str = "f32", epsilon: float = 0.05, use_graph: bool = True, blocks=None, start_goal=None):
+                 dtype: str = "f32", epsilon: float = 0.05, use_graph: bool = True, blocks=None, start_goal=None,
+                 rollouts: str = "jointspace"):
         import torch
         self.torch = torch
+        if rollouts not in ROLLOUT_MODELS:
+            raise MrfError(f"rollouts must be one of {sorted(ROLLOUT_MODELS)}, got {rollouts!r}")
+        if rollouts == "cartesian" and not rollout_fabrics:
+            raise MrfError('rollouts="cartesian" needs rollout_fabrics=True (MRDF runs no rollouts)')
+        self.rollout_model = ROLLOUT_MODELS[rollouts]
         B, R, _ = rec.shape
         self.B, self.R, self.N = B, R, int(n_horizon)
         self.rollout_fabrics, self.resolve_deadlocks = rollout_fabrics, resolve_deadlocks
         self.n_per_link, self.epsilon, self.use_graph = int(n_obst_per_link), float(epsilon), use_graph
         self.dev = torch.device(f"cuda:{device}")
         self.tdt = torch.float32 if dtype == "f32" else torch.float64
-        self.fab = Fabrics(R, device=device, estimate_goal=1 if estimate_goal else 0, static_or_dyn=static_or_dyn)
+        # RF-CV goal estimate: Jacobian column 0 in the joint-space example (:346-348), J qdot in the Cartesian one (:355-357)
+        est_mode = (2 if self.rollout_model == 1 else 1) if estimate_goal else 0
+        self.fab = Fabrics(R, device=device, estimate_goal=est_mode, static_or_dyn=static_or_dyn)
         self.fab.handle.set_coop_max_batch(0 if B > 256 else 1 << 20)
         t = lambda a, dt=None: torch.from_numpy(np.ascontiguousarray(a)).to(self.dev, dtype=dt or self.tdt)
         self.rec = t(to_soa(rec))                                    # (44,R,B): q, qdot rows are the live state
@@ -75,6 +96,8 @@ class BatchedEpisodes:
             self.goal0.copy_(self.start_goal)                                         # :33
             self.w0.fill_(2.0)                                                        # :34
             self.kin_scratch = z(3, 8, 3, R, B)
+        if self.rollout_model == 1 and not self.pick_and_place:
+            self.kin_scratch = z(3, 8, 3, R, B)                                       # hand FK and J qdot
         self.graph = None
         self.steps_done = 0
         self._ep = None
@@ -91,7 +114,9 @@ class BatchedEpisodes:
         ep = MrfEpisode()
         ep.struct_size = C.sizeof(MrfEpisode)
         ep.n_horizon, ep.rollout_fabrics, ep.resolve_deadlocks = self.N, int(self.rollout_fabrics), int(self.resolve_deadlocks)
-        ep.n_per_link, ep.epsilon, ep.w1_rollout, ep.w1_action, ep.clearance_radius_sum = self.n_per_link, self.epsilon, 10.0, 20.0, 0.16
+        ep.rollout_model = self.rollout_model
+        w1_rollout = 20.0 if self.rollout_model == 1 else 10.0          # example_pandas_cartesian.py:42 / _Jointspace.py:43
+        ep.n_per_link, ep.epsilon, ep.w1_rollout, ep.w1_action, ep.clearance_radius_sum = self.n_per_link, self.epsilon, w1_rollout, 20.0, 0.16
         for i, v in enumerate(VEL_LIMITS):
             ep.vel_limit[i] = v
         ep.offsets = self._offsets.ctypes.data
