@@ -28,6 +28,7 @@
  *                         multi_robot_fabrics/utils/utils.py:87-119, utils/utils_apply_fk.py:3-33,
  *                         examples/example_pandas_Jointspace.py:400-412
  *   mrf_point_action_*    point-mass planner compute_action (examples/example_pointmasses_static.py:102-129,191-199)
+ *   mrf_point_episode_run_* the control loops of examples/example_pointmasses_static.py and _dynamic.py, many steps per call
  *   mrf_fsm_*             StateMachine.get_state_machine_panda + gripper action
  *                         multi_robot_fabrics/others_planner/state_machine.py:70-84,133-214
  *   mrf_episode_step_*    one iteration of the control loop examples/example_pandas_Jointspace.py:280-458 (coupled
@@ -63,6 +64,7 @@ extern "C" {
 #define MRF_GUARD_SLOTS 8   /* scratch slots of the mrf_rfcv_post_dev_f32 re-roll (concurrent post steps on different streams) */
 #define MRF_MAX_STATIC 16   /* static spheres per robot in a coupled rollout (nr_obsts of the rollout planners) */
 #define MRF_MAX_SPHERES_PER_LINK 8   /* n_obst_per_link, examples/configs/panda_config.yaml:8 (reference default 4) */
+#define MRF_MAX_POINT_ROBOTS 8   /* point robots per scenario in mrf_point_episode_run_dev_* */
 
 /* Per-robot record = the numeric arguments of one fabric action / of get_velocity_rollouts
  * (forward_planner_Jointspace.py:303-329), fixed order:
@@ -416,6 +418,47 @@ typedef struct MrfEpisode {
 } MrfEpisode;
 int mrf_episode_step_dev_f64(mrf_handle_t h, const MrfEpisode* ep, int64_t B, void* stream);
 int mrf_episode_step_dev_f32(mrf_handle_t h, const MrfEpisode* ep, int64_t B, void* stream);
+
+/* Closed-loop point-mass episodes of B independent scenarios, n_steps control steps in ONE launch: the control loops of
+ * examples/example_pointmasses_static.py (dynamic = 0) and examples/example_pointmasses_dynamic.py (dynamic = 1) with a
+ * kinematic environment.  Per step, for every robot i of every scenario, all robots reading the state at the start of
+ * the step (Jacobi order):
+ *   1. metrics of the measured state: done_at = first time_step at which every robot is within `epsilon` of its goal in
+ *      (x, y); running minima of the x-y robot-robot clearance |p_i - p_j| - (r_i + r_j) and of the robot-scene clearance
+ *      |(x, y, 0.05) - c_o| - (r_o + r_i) (the distance the collision leaf sees).
+ *   2. obstacles of robot i: the n_scene scene spheres, then the other robots ascending.  Static variant: robot j is a
+ *      static sphere at its full joint position q_j = (x, y, theta), radius r_j -- the third component lands in the
+ *      sphere's z, a quirk of the reference's static example kept as is (theta is only ever damped).  Dynamic variant:
+ *      robot j is a 2-D sphere at q_j[0:2] with velocity qdot_j[0:2], acceleration 0, radius r_j.
+ *   3. action: the planner of mrf_point_action_dev_* (mode 'acc', one 2-D goal, eps / jdot_sign / exec_scale of the
+ *      handle's MrfConfig).  compute_action's |a| < 1e-6 zeroing is not applied (neither does mrf_episode_step_dev_*).
+ *   4. environment: a non-finite action becomes 0 for the step, which is counted in nonfinite_steps; then
+ *      qdot += dt a, q += dt qdot (semi-implicit Euler, dt = MrfConfig.dt, each product and sum rounded on its own).
+ *      ASSUMPTION: urdfenvs integrates a commanded velocity through its velocity controller; this kinematic double
+ *      integrator stands in for its acceleration mode.
+ * No rollouts and no deadlock logic (the reference's point examples run neither).  Splitting an episode over several
+ * calls (n_steps each) gives the same bits as one call.  Device pointers of the entry's precision T unless typed, b
+ * fastest. */
+typedef struct MrfPointEpisode {
+    int32_t struct_size;        /* sizeof(MrfPointEpisode) */
+    int32_t n_robots;           /* R, 2..MRF_MAX_POINT_ROBOTS */
+    int32_t dynamic;            /* 0: other robots are static spheres (static example), 1: dynamic 2-D spheres */
+    int32_t n_scene;            /* scene spheres per scenario, 0..MRF_MAX_STATIC */
+    double epsilon;             /* reach tolerance in (x, y) */
+    void* state;                /* T [6][R][B] in/out: q (x, y, theta), qdot */
+    const void* goal;           /* T [R][2][B] */
+    const void* weight;         /* T [R][B] weight_goal_0 */
+    const void* radius;         /* T [R][B] radius_body_base_link */
+    const void* scene;          /* T [n_scene][4][B] x, y, z, radius (nullable when n_scene = 0) */
+    int32_t* time_step;         /* [B] in/out, += n_steps */
+    int32_t* done_at;           /* [B] in/out (-1 = not yet) */
+    int32_t* nonfinite_steps;   /* [B] in/out */
+    void* min_clear_robots;     /* T [B] in/out: running minimum */
+    void* min_clear_scene;      /* T [B] in/out: running minimum */
+    void* traj;                 /* T [n_steps][3][R][B] out, nullable: q after each step of this call */
+} MrfPointEpisode;
+int mrf_point_episode_run_dev_f64(mrf_handle_t h, const MrfPointEpisode* ep, int64_t B, int32_t n_steps, void* stream);
+int mrf_point_episode_run_dev_f32(mrf_handle_t h, const MrfPointEpisode* ep, int64_t B, int32_t n_steps, void* stream);
 
 /* mrf_rollout_* picks between two kernels computing the same recurrence: the cooperative low-latency kernel (one CTA
  * per scenario, one warp per robot) for B <= max_batch, the throughput kernel (one thread per scenario and robot)

@@ -57,6 +57,17 @@ class MrfEpisode(C.Structure):
     ]
 
 
+class MrfPointEpisode(C.Structure):
+    """include/mrf_b200.h: state of mrf_point_episode_run_dev_* (device pointers as integers)."""
+    _fields_ = [
+        ("struct_size", C.c_int32), ("n_robots", C.c_int32), ("dynamic", C.c_int32), ("n_scene", C.c_int32),
+        ("epsilon", C.c_double), ("state", C.c_void_p), ("goal", C.c_void_p), ("weight", C.c_void_p),
+        ("radius", C.c_void_p), ("scene", C.c_void_p), ("time_step", C.c_void_p), ("done_at", C.c_void_p),
+        ("nonfinite_steps", C.c_void_p), ("min_clear_robots", C.c_void_p), ("min_clear_scene", C.c_void_p),
+        ("traj", C.c_void_p),
+    ]
+
+
 _lib = None
 _F = {"f32": (C.c_float, np.float32), "f64": (C.c_double, np.float64)}
 
@@ -75,7 +86,7 @@ EXPORTS = [
     "mrf_rollout_host_submit_compact_f64", "mrf_rollout_host_submit_compact_f32",
     "mrf_rfcv_post_dev_f32", "mrf_rfcv_post_dev_f64", "mrf_rollout_risk_dev_f32", "mrf_rollout_risk_dev_f64",
     "mrf_set_guard", "mrf_guard_stats", "mrf_rollout_static_dev_f32", "mrf_rollout_static_dev_f64",
-    "mrf_rfcv_host_submit_f32",
+    "mrf_rfcv_host_submit_f32", "mrf_point_episode_run_dev_f64", "mrf_point_episode_run_dev_f32",
 ]
 
 
@@ -130,6 +141,8 @@ def lib():
     L.mrf_rollout_host_submit_compact_f32.argtypes = [vp, vp, vp, i32, vp, vp, vp, i64]
     L.mrf_episode_step_dev_f64.argtypes = [vp, C.POINTER(MrfEpisode), i64, vp]
     L.mrf_episode_step_dev_f32.argtypes = [vp, C.POINTER(MrfEpisode), i64, vp]
+    L.mrf_point_episode_run_dev_f64.argtypes = [vp, C.POINTER(MrfPointEpisode), i64, i32, vp]
+    L.mrf_point_episode_run_dev_f32.argtypes = [vp, C.POINTER(MrfPointEpisode), i64, i32, vp]
     L.mrf_fma_peak.argtypes = [vp, i32, C.POINTER(C.c_double)]
     _lib = L
     return L

@@ -794,30 +794,16 @@ __global__ void __launch_bounds__(kActThreads)
 //   rec [10][B]: q[3], qdot[3], x_goal_0[2], weight_goal_0, radius_body_base_link
 //   stat [Ss][4][B]: x[3], radius          dyn [Sd][7][B]: x[2], xdot[2], xddot[2], radius
 // ------------------------------------------------------------------------------------------------
-template <typename T>
-__global__ void __launch_bounds__(kActThreads)
-    point_action_kernel(T eps, T sigma, T s2, const T* __restrict__ rec, int Ss, const T* __restrict__ stat, int Sd,
-                        const T* __restrict__ dyn, T* __restrict__ action, long long B) {
-    const long long b = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (b >= B) return;
-    auto ld = [&](int f) { return rec[(long long)f * B + b]; };
-    const T qx = ld(0), qy = ld(1), vx = ld(3), vy = ld(4), vth = ld(5);
-    const T gx = ld(6), gy = ld(7), wg = ld(8), rb = ld(9);
+// point_action: the planner for one robot with ego state (qx, qy, theta), (vx, vy, vth), goal (gx, gy), weight wg.
+// `each(leaf)` enumerates the obstacle spheres in order, calling leaf(dx, dy, dz, wx, wy, ax, ay, rho) with the offset
+// ego - obstacle, the relative velocity, the obstacle's acceleration and rho = radius_obst + radius_body.  Writes the
+// action (a0, a1, a2).  Shared by point_action_kernel (obstacles from global memory) and point_episode_kernel (scene
+// spheres from shared memory, other robots from neighbouring lanes).
+template <typename T, typename Each>
+__device__ __forceinline__ void point_action(T eps, T sigma, T s2, T qx, T qy, T vx, T vy, T vth, T gx, T gy, T wg, Each each,
+                                             T& a0, T& a1, T& a2) {
     T m00 = T(0.2), m01 = T(0), m11 = T(0.2), f0 = T(0), f1 = T(0), num = T(0);
-    for (int o = 0; o < Ss + Sd; ++o) {
-        T dx, dy, dz, wx, wy, ax = T(0), ay = T(0), rho;
-        if (o < Ss) {
-            const T* p = stat + (long long)o * 4 * B + b;
-            dx = qx - p[0]; dy = qy - p[B]; dz = T(0.05) - p[2 * B];
-            wx = vx; wy = vy;
-            rho = p[3 * B] + rb;
-        } else {
-            const T* p = dyn + (long long)(o - Ss) * 7 * B + b;
-            dx = qx - p[0]; dy = qy - p[B]; dz = T(0);
-            wx = vx - p[2 * B]; wy = vy - p[3 * B];
-            ax = p[4 * B]; ay = p[5 * B];
-            rho = p[6 * B] + rb;
-        }
+    each([&](T dx, T dy, T dz, T wx, T wy, T ax, T ay, T rho) {
         const T n2 = dx * dx + dy * dy + dz * dz;
         const T in1 = Mth<T>::rsqrt(n2), n = n2 * in1;
         const T t = n - rho, nr = n * rho, u = Mth<T>::rcp(nr * t);
@@ -835,7 +821,7 @@ __global__ void __launch_bounds__(kActThreads)
         f0 += g0 * fq; f1 += g1 * fq;
         m00 += Ml * g0 * g0; m01 += Ml * g0 * g1; m11 += Ml * g1 * g1;
         num += (g0 * vx + g1 * vy) * (fq - feq);
-    }
+    });
     const T xg0 = qx - gx, xg1 = qy - gy;
     const T ng = Mth<T>::sqrt(xg0 * xg0 + xg1 * xg1);
     T dpsi, mm;
@@ -860,9 +846,156 @@ __global__ void __launch_bounds__(kActThreads)
     const T beta = T(0.5) * (Mth<T>::tanh(T(-0.5) * (ng - T(0.02))) + T(1)) * T(6.5) + T(0.01) +
                    Mth<T>::max(T(0), a_geom - a_ex);
     const T damp = a_ex + beta;
-    action[b] = -hf0 - damp * vx;
-    action[B + b] = -hf1 - damp * vy;
-    action[2 * B + b] = -damp * vth;
+    a0 = -hf0 - damp * vx;
+    a1 = -hf1 - damp * vy;
+    a2 = -damp * vth;
+}
+
+template <typename T>
+__global__ void __launch_bounds__(kActThreads)
+    point_action_kernel(T eps, T sigma, T s2, const T* __restrict__ rec, int Ss, const T* __restrict__ stat, int Sd,
+                        const T* __restrict__ dyn, T* __restrict__ action, long long B) {
+    const long long b = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (b >= B) return;
+    auto ld = [&](int f) { return rec[(long long)f * B + b]; };
+    const T qx = ld(0), qy = ld(1), vx = ld(3), vy = ld(4), vth = ld(5);
+    const T gx = ld(6), gy = ld(7), wg = ld(8), rb = ld(9);
+    auto each = [&](auto&& leaf) {
+        for (int o = 0; o < Ss + Sd; ++o) {
+            T dx, dy, dz, wx, wy, ax = T(0), ay = T(0), rho;
+            if (o < Ss) {
+                const T* p = stat + (long long)o * 4 * B + b;
+                dx = qx - p[0]; dy = qy - p[B]; dz = T(0.05) - p[2 * B];
+                wx = vx; wy = vy;
+                rho = p[3 * B] + rb;
+            } else {
+                const T* p = dyn + (long long)(o - Ss) * 7 * B + b;
+                dx = qx - p[0]; dy = qy - p[B]; dz = T(0);
+                wx = vx - p[2 * B]; wy = vy - p[3 * B];
+                ax = p[4 * B]; ay = p[5 * B];
+                rho = p[6 * B] + rb;
+            }
+            leaf(dx, dy, dz, wx, wy, ax, ay, rho);
+        }
+    };
+    T a0, a1, a2;
+    point_action<T>(eps, sigma, s2, qx, qy, vx, vy, vth, gx, gy, wg, each, a0, a1, a2);
+    action[b] = a0;
+    action[B + b] = a1;
+    action[2 * B + b] = a2;
+}
+
+// ------------------------------------------------------------------------------------------------
+// closed-loop point-mass episodes (examples/example_pointmasses_static.py, _dynamic.py), many control steps per launch.
+// thread = (scenario, robot): the R robots of a scenario sit in W consecutive lanes (W = R rounded up to a power of two,
+// lanes R..W-1 idle) and read each other's state by __shfl_sync(..., W).  q, qdot and the running metrics stay in
+// registers for the whole launch; the scenario's scene spheres are staged once in shared memory.  Per step, every
+// robot i of every scenario at once, all robots reading the state at the start of the step:
+//   metrics of the measured state: reached (every robot within eps_goal of its goal in x-y; done_at = first such step),
+//     x-y robot-robot clearance |p_i - p_j| - (r_i + r_j), scene clearance |(x, y, 0.05) - c_o| - (r_o + r_i)
+//   obstacles: the scene spheres, then the other robots ascending -- DYN = false: a static sphere at q_j = (x, y, theta)
+//     of radius r_j (the reference's static example passes the whole joint vector, so theta lands in the sphere's z;
+//     theta is only ever damped); DYN = true: a 2-D sphere at q_j[0:2] moving with qdot_j[0:2], no acceleration
+//   action: point_action (the planner of mrf_point_action_dev)
+//   environment: a non-finite action becomes 0 for the step and the step is counted; qdot += dt a, q += dt qdot
+//     (semi-implicit Euler, every product and sum rounded on its own: no FMA contraction)
+// The one barrier (scene staging) comes before any per-lane branch, so a scenario's bits never depend on its neighbours.
+// ------------------------------------------------------------------------------------------------
+constexpr int kPointThreads = 128;
+
+template <typename T> __device__ __forceinline__ T mul_rn(T a, T b);
+template <> __device__ __forceinline__ float mul_rn(float a, float b) { return __fmul_rn(a, b); }
+template <> __device__ __forceinline__ double mul_rn(double a, double b) { return __dmul_rn(a, b); }
+template <typename T> __device__ __forceinline__ T add_rn(T a, T b);
+template <> __device__ __forceinline__ float add_rn(float a, float b) { return __fadd_rn(a, b); }
+template <> __device__ __forceinline__ double add_rn(double a, double b) { return __dadd_rn(a, b); }
+
+template <typename T, bool DYN>
+__global__ void __launch_bounds__(kPointThreads)
+    point_episode_kernel(T eps, T sigma, T s2, T dt, T eps_goal, int R, int W, int n_scene, int n_steps,
+                         T* __restrict__ state, const T* __restrict__ goal, const T* __restrict__ weight,
+                         const T* __restrict__ radius, const T* __restrict__ scene, int32_t* __restrict__ time_step,
+                         int32_t* __restrict__ done_at, int32_t* __restrict__ nonfinite, T* __restrict__ min_rr,
+                         T* __restrict__ min_sc, T* __restrict__ traj, long long B) {
+    extern __shared__ __align__(16) unsigned char point_smem[];
+    T* sc = reinterpret_cast<T*>(point_smem);        // [spb][n_scene][4]
+    const int spb = blockDim.x / W, g = threadIdx.x / W, i = threadIdx.x % W;
+    const long long b0 = (long long)blockIdx.x * spb, b = b0 + g;
+    const int nf = n_scene * 4;
+    for (int k = threadIdx.x; k < spb * nf; k += blockDim.x) { // scenario fastest: coalesced reads
+        const int s = k % spb, f = k / spb;
+        sc[s * nf + f] = b0 + s < B ? scene[(long long)f * B + b0 + s] : T(0);
+    }
+    __syncthreads();
+    const bool live = b < B && i < R;
+    const long long RB = (long long)R * B, idx = (long long)i * B + b;
+    T qx = T(0), qy = T(0), qt = T(0), vx = T(0), vy = T(0), vt = T(0), gx = T(0), gy = T(0), wg = T(0), rb = T(0);
+    if (live) {
+        qx = state[idx]; qy = state[RB + idx]; qt = state[2 * RB + idx];
+        vx = state[3 * RB + idx]; vy = state[4 * RB + idx]; vt = state[5 * RB + idx];
+        gx = goal[((long long)i * 2) * B + b]; gy = goal[((long long)i * 2 + 1) * B + b];
+        wg = weight[idx]; rb = radius[idx];
+    }
+    int t0 = 0, done = -1, nbad = 0;
+    if (b < B) { t0 = time_step[b]; done = done_at[b]; nbad = nonfinite[b]; }
+    const T inf = T(INFINITY);
+    T mrr = inf, msc = inf;                          // this robot's running minima; reduced over the group at the end
+    const unsigned gmask = ((1u << R) - 1u) << ((threadIdx.x & 31) & ~(W - 1));
+    const T* my_sc = sc + g * nf;
+    for (int k = 0; k < n_steps; ++k) {
+        const T ex = qx - gx, ey = qy - gy;
+        const unsigned near = __ballot_sync(0xffffffffu, Mth<T>::sqrt(ex * ex + ey * ey) < eps_goal);
+        if ((near & gmask) == gmask && done < 0) done = t0 + k;
+        auto each = [&](auto&& leaf) {
+            for (int o = 0; o < n_scene; ++o) {
+                const T* p = my_sc + o * 4;
+                const T dx = qx - p[0], dy = qy - p[1], dz = T(0.05) - p[2], rho = p[3] + rb;
+                const T c = Mth<T>::sqrt(dx * dx + dy * dy + dz * dz) - rho;
+                msc = c < msc ? c : msc;
+                leaf(dx, dy, dz, vx, vy, T(0), T(0), rho);
+            }
+            for (int j = 0; j < R; ++j) { // every lane shuffles (uniform trip count); the leaf skips robot i itself
+                const T xj = __shfl_sync(0xffffffffu, qx, j, W), yj = __shfl_sync(0xffffffffu, qy, j, W);
+                const T rj = __shfl_sync(0xffffffffu, rb, j, W);
+                const T uj = __shfl_sync(0xffffffffu, DYN ? vx : qt, j, W); // DYN: x-velocity of robot j, else its theta
+                const T wj = DYN ? __shfl_sync(0xffffffffu, vy, j, W) : T(0);
+                if (j == i) continue;
+                const T dx = qx - xj, dy = qy - yj, rho = rj + rb;
+                const T c = Mth<T>::sqrt(dx * dx + dy * dy) - rho;
+                mrr = c < mrr ? c : mrr;
+                if (DYN) leaf(dx, dy, T(0), vx - uj, vy - wj, T(0), T(0), rho);
+                else leaf(dx, dy, T(0.05) - uj, vx, vy, T(0), T(0), rho);
+            }
+        };
+        T a0, a1, a2;
+        point_action<T>(eps, sigma, s2, qx, qy, vx, vy, vt, gx, gy, wg, each, a0, a1, a2);
+        const bool bad = !(a0 - a0 == T(0) && a1 - a1 == T(0) && a2 - a2 == T(0));
+        if (bad) { a0 = T(0); a1 = T(0); a2 = T(0); }
+        if (__ballot_sync(0xffffffffu, bad) & gmask) ++nbad;
+        vx = add_rn(vx, mul_rn(dt, a0)); vy = add_rn(vy, mul_rn(dt, a1)); vt = add_rn(vt, mul_rn(dt, a2));
+        qx = add_rn(qx, mul_rn(dt, vx)); qy = add_rn(qy, mul_rn(dt, vy)); qt = add_rn(qt, mul_rn(dt, vt));
+        if (traj != nullptr && live) {
+            T* p = traj + (long long)k * 3 * RB + idx;
+            p[0] = qx; p[RB] = qy; p[2 * RB] = qt;
+        }
+    }
+    if (!live) { mrr = inf; msc = inf; }
+    for (int off = W / 2; off > 0; off >>= 1) { // min is exact: the order of the reduction does not matter
+        const T orr = __shfl_xor_sync(0xffffffffu, mrr, off, W), osc = __shfl_xor_sync(0xffffffffu, msc, off, W);
+        mrr = orr < mrr ? orr : mrr;
+        msc = osc < msc ? osc : msc;
+    }
+    if (live) {
+        state[idx] = qx; state[RB + idx] = qy; state[2 * RB + idx] = qt;
+        state[3 * RB + idx] = vx; state[4 * RB + idx] = vy; state[5 * RB + idx] = vt;
+    }
+    if (b < B && i == 0) {
+        time_step[b] = t0 + n_steps;
+        done_at[b] = done;
+        nonfinite[b] = nbad;
+        if (mrr < min_rr[b]) min_rr[b] = mrr;
+        if (msc < min_sc[b]) min_sc[b] = msc;
+    }
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -2414,6 +2547,41 @@ extern "C" int mrf_point_action_host_f64(mrf_handle_t h, const double* rec, int 
     rc = download_aos<double>(h, action, B, 3, 6, 7);
     if (rc) return rc;
     return finish_timed(h);
+}
+
+template <typename T>
+static int point_episode_run_dev(mrf_handle_t h, const MrfPointEpisode* ep, int64_t B, int32_t n_steps, void* stream) {
+    if (!h || !ep) return fail(MRF_EINVAL, "mrf_point_episode_run: null argument");
+    if (ep->struct_size != (int32_t)sizeof(MrfPointEpisode))
+        return fail(MRF_EINVAL, "mrf_point_episode_run: MrfPointEpisode size mismatch");
+    const int R = ep->n_robots;
+    if (R < 2 || R > MRF_MAX_POINT_ROBOTS) return fail(MRF_EINVAL, "mrf_point_episode_run: n_robots must be 2..MRF_MAX_POINT_ROBOTS");
+    if (ep->n_scene < 0 || ep->n_scene > MRF_MAX_STATIC) return fail(MRF_EINVAL, "mrf_point_episode_run: n_scene must be 0..MRF_MAX_STATIC");
+    if (ep->dynamic != 0 && ep->dynamic != 1) return fail(MRF_EINVAL, "mrf_point_episode_run: dynamic must be 0 or 1");
+    if (!ep->state || !ep->goal || !ep->weight || !ep->radius || (ep->n_scene > 0 && !ep->scene) || !ep->time_step ||
+        !ep->done_at || !ep->nonfinite_steps || !ep->min_clear_robots || !ep->min_clear_scene)
+        return fail(MRF_EINVAL, "mrf_point_episode_run: null state pointer");
+    if (B <= 0) return fail(MRF_EINVAL, "mrf_point_episode_run: B must be positive");
+    if (n_steps < 1) return fail(MRF_EINVAL, "mrf_point_episode_run: n_steps must be positive");
+    MRF_CUDA(cudaSetDevice(h->device));
+    const int W = R <= 2 ? 2 : (R <= 4 ? 4 : 8), spb = kPointThreads / W;
+    const unsigned grid = (unsigned)((B + spb - 1) / spb);
+    const size_t smem = sizeof(T) * (size_t)spb * ep->n_scene * 4;
+    auto kern = ep->dynamic ? point_episode_kernel<T, true> : point_episode_kernel<T, false>;
+    kern<<<grid, kPointThreads, smem, (cudaStream_t)stream>>>(
+        (T)h->cfg.eps, (T)h->cfg.jdot_sign, (T)(2.0 * h->cfg.exec_scale), (T)h->cfg.dt, (T)ep->epsilon, R, W, ep->n_scene,
+        n_steps, (T*)ep->state, (const T*)ep->goal, (const T*)ep->weight, (const T*)ep->radius, (const T*)ep->scene,
+        ep->time_step, ep->done_at, ep->nonfinite_steps, (T*)ep->min_clear_robots, (T*)ep->min_clear_scene, (T*)ep->traj,
+        (long long)B);
+    MRF_CUDA(cudaGetLastError());
+    h->launches += 1;
+    return MRF_OK;
+}
+extern "C" int mrf_point_episode_run_dev_f64(mrf_handle_t h, const MrfPointEpisode* ep, int64_t B, int32_t n_steps, void* stream) {
+    return point_episode_run_dev<double>(h, ep, B, n_steps, stream);
+}
+extern "C" int mrf_point_episode_run_dev_f32(mrf_handle_t h, const MrfPointEpisode* ep, int64_t B, int32_t n_steps, void* stream) {
+    return point_episode_run_dev<float>(h, ep, B, n_steps, stream);
 }
 
 template <typename T>

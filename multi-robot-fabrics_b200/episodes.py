@@ -27,6 +27,9 @@ Two rollout models (`rollouts=`).  "jointspace" (default) is the loop above: cou
   5.-6. obstacle staging with link-origin velocities, executed action, integration: as in the joint-space loop
      (the Cartesian example's action-side staging is taken to be the joint-space example's).
 The rollouts always use the planner with collision links (no grasp planner inside the horizon), as the coupled ones do.
+
+BatchedPointEpisodes runs the loops of the two point-mass examples (examples/example_pointmasses_static.py, _dynamic.py):
+many control steps per kernel launch, see its docstring.
 """
 from __future__ import annotations
 
@@ -179,3 +182,104 @@ class BatchedEpisodes:
                 "q": self.rec[Q:Q + 7].permute(2, 1, 0).double().cpu().numpy(),
                 "x_ee": (self.xee.permute(2, 0, 1) if (self.rollout_fabrics or self.pick_and_place) else
                          self.kin_scratch[0, 7].permute(2, 1, 0)).double().cpu().numpy()}
+
+
+class BatchedPointEpisodes:
+    """Closed-loop point-mass episodes: the control loops of examples/example_pointmasses_static.py (dynamic=False) and
+    examples/example_pointmasses_dynamic.py (dynamic=True) for B independent scenarios of R = 2..8 point robots (3 dof:
+    x, y, theta), entirely on the GPU.  Every call of run(n) is ONE C-ABI call, mrf_point_episode_run_dev_*, that runs n
+    control steps in one kernel launch with the state in registers; the loop itself (obstacles, planner, integration,
+    metrics) is documented at MrfPointEpisode in include/mrf_b200.h.  Splitting an episode over several run() calls
+    gives the same bits as one call.
+
+      q0 (B,R,3), goals (B,R,2), scene (B,S,4) x, y, z, radius of S <= 16 scene spheres (or None), radius / weight:
+      body radius and weight_goal_0 (scalars or (B,R)), qdot0 (B,R,3) (default 0).
+    An episode succeeds when every robot is within `epsilon` of its goal in (x, y).  The reference's point examples do
+    not record a goal tolerance; the default 0.05 is the Panda loop's (BatchedEpisodes).  dt and the planner constants
+    come from default_config(1), the handle PointFabricPlanner uses.
+    """
+
+    def __init__(self, q0, goals, scene=None, dynamic: bool = False, radius=0.2, weight=1.0, qdot0=None,
+                 epsilon: float = 0.05, dtype: str = "f32", device: int = 0, record: bool = False):
+        import torch
+        from ._lib import default_config
+        self.torch = torch
+        q0 = np.asarray(q0, dtype=np.float64)
+        if q0.ndim != 3 or q0.shape[2] != 3:
+            raise MrfError(f"q0 must be (B, R, 3), got {q0.shape}")
+        B, R, _ = q0.shape
+        goals = np.asarray(goals, dtype=np.float64)
+        if goals.shape != (B, R, 2):
+            raise MrfError(f"goals must be ({B}, {R}, 2), got {goals.shape}")
+        scene = np.zeros((B, 0, 4)) if scene is None else np.asarray(scene, dtype=np.float64)
+        if scene.ndim != 3 or scene.shape[0] != B or scene.shape[2] != 4:
+            raise MrfError(f"scene must be ({B}, S, 4), got {scene.shape}")
+        qdot0 = np.zeros((B, R, 3)) if qdot0 is None else np.asarray(qdot0, dtype=np.float64)
+        if qdot0.shape != (B, R, 3):
+            raise MrfError(f"qdot0 must be ({B}, {R}, 3), got {qdot0.shape}")
+        if dtype not in ("f32", "f64"):
+            raise MrfError(f"dtype must be 'f32' or 'f64', got {dtype!r}")
+        self.B, self.R, self.S = B, R, scene.shape[1]
+        self.dynamic, self.epsilon, self.record = bool(dynamic), float(epsilon), bool(record)
+        self.dev = torch.device(f"cuda:{device}")
+        self.tdt = torch.float32 if dtype == "f32" else torch.float64
+        self.fab = Fabrics(config=default_config(1), device=device)
+        t = lambda a: torch.from_numpy(np.ascontiguousarray(a)).to(self.dev, dtype=self.tdt)
+        self.state = t(np.concatenate([q0, qdot0], axis=2).transpose(2, 1, 0))              # (6,R,B)
+        self.goal = t(goals.transpose(1, 2, 0))                                             # (R,2,B)
+        self.weight = t(np.broadcast_to(np.asarray(weight, dtype=np.float64), (B, R)).T)    # (R,B)
+        self.radius = t(np.broadcast_to(np.asarray(radius, dtype=np.float64), (B, R)).T)    # (R,B)
+        self.scene = t(scene.transpose(1, 2, 0)) if self.S else None                       # (S,4,B)
+        i32 = lambda v: torch.full((B,), v, dtype=torch.int32, device=self.dev)
+        self.time_step, self.done_at, self.nonfinite_steps = i32(0), i32(-1), i32(0)
+        self.min_clear_robots = torch.full((B,), float("inf"), dtype=self.tdt, device=self.dev)
+        self.min_clear_scene = torch.full((B,), float("inf"), dtype=self.tdt, device=self.dev)
+        self.traj = []                                                                      # (n,3,R,B) per run()
+        self.steps_done = 0
+        self._ep = None
+
+    def _episode_struct(self):
+        """The MrfPointEpisode argument of mrf_point_episode_run_dev_* (built once: the state tensors never move)."""
+        import ctypes as C
+        from ._lib import MrfPointEpisode
+        ep = MrfPointEpisode()
+        ep.struct_size = C.sizeof(MrfPointEpisode)
+        ep.n_robots, ep.dynamic, ep.n_scene, ep.epsilon = self.R, int(self.dynamic), self.S, self.epsilon
+        p = lambda t: None if t is None else t.data_ptr()
+        ep.state, ep.goal, ep.weight, ep.radius, ep.scene = p(self.state), p(self.goal), p(self.weight), p(self.radius), p(self.scene)
+        ep.time_step, ep.done_at, ep.nonfinite_steps = p(self.time_step), p(self.done_at), p(self.nonfinite_steps)
+        ep.min_clear_robots, ep.min_clear_scene = p(self.min_clear_robots), p(self.min_clear_scene)
+        return ep
+
+    def run(self, n_steps: int):
+        """n_steps control steps in one kernel launch on torch's current stream."""
+        import ctypes as C
+        from ._lib import check, lib
+        if self._ep is None:
+            self._ep = self._episode_struct()
+        n_steps = int(n_steps)
+        traj = None
+        if self.record and n_steps > 0:
+            traj = self.torch.empty((n_steps, 3, self.R, self.B), dtype=self.tdt, device=self.dev)
+            self.traj.append(traj)
+        self._ep.traj = None if traj is None else traj.data_ptr()
+        fn = lib().mrf_point_episode_run_dev_f32 if self.tdt == self.torch.float32 else lib().mrf_point_episode_run_dev_f64
+        check(fn(self.fab.handle.ptr, C.byref(self._ep), self.B, n_steps, self.torch.cuda.current_stream(self.dev).cuda_stream),
+              "mrf_point_episode_run_dev")
+        self.steps_done += n_steps
+        return self
+
+    def results(self) -> dict:
+        """success, steps_to_success (-1 = not reached), min_clear_robots / min_clear_scene (running minima), nonfinite_steps
+        (B,); q, qdot (B,R,3); traj (B,T,R,3), q after each step, when recorded."""
+        self.torch.cuda.synchronize(self.dev)
+        done = self.done_at.cpu().numpy()
+        st = self.state.permute(2, 1, 0).double().cpu().numpy()                             # (B,R,6)
+        out = {"steps": self.steps_done, "success": done >= 0, "steps_to_success": done,
+               "min_clear_robots": self.min_clear_robots.double().cpu().numpy(),
+               "min_clear_scene": self.min_clear_scene.double().cpu().numpy(),
+               "nonfinite_steps": self.nonfinite_steps.cpu().numpy(), "q": st[:, :, 0:3], "qdot": st[:, :, 3:6]}
+        if self.record:
+            tr = self.torch.cat(self.traj) if self.traj else self.torch.empty((0, 3, self.R, self.B), dtype=self.tdt)
+            out["traj"] = tr.permute(3, 0, 2, 1).double().cpu().numpy()
+        return out

@@ -133,3 +133,67 @@ def pick_and_place_layout(rec: np.ndarray, n_blocks: int = 2, seed: int = 0, spr
                                               rng.uniform(-spread, spread, (B, n_blocks, R)),
                                               np.full((B, n_blocks, R), -drop)], axis=-1)
     return blocks, start
+
+
+# ---- point masses (examples/example_pointmasses_static.py, _dynamic.py): 4 point robots swap sides between 6 spheres
+POINT_SCENE = np.array([[1, 1.25, 0], [1, 3.75, 0], [1, -1.25, 0], [-1.1, 0, 0], [-1.1, 2.5, 0], [-1.1, -2.5, 0]], float)
+POINT_SCENE_RADIUS = 1.0
+POINT_STARTS = np.array([[-2.5, 0.01, 0.0], [-2.5, -2.49, 0.0], [2.5, 1.26, 0.0], [2.5, 3.74, 0.0]])
+POINT_GOALS = np.array([[1.5, 3.76], [1.5, 1.26], [-2.5, 0.01], [-2.5, -2.49]])
+POINT_RADIUS = 0.2
+
+
+def point_masses(B: int, seed: int = 0, jitter: float = 0.0):
+    """The point-mass examples' scene for episodes.BatchedPointEpisodes: 6 scene spheres of radius 1.0, 4 robots of radius
+    0.2 and their start / goal swap pairs.  With jitter > 0 every scenario's starts and goals move by uniform offsets in
+    [-jitter, jitter] in x and y (PCG64(seed)); a draw whose start has a robot in contact with another robot (x-y) or with
+    a scene sphere (the collision leaf's distance from (x, y, 0.05)) is redrawn.  jitter = 0 is the example itself.
+    -> q0 (B,4,3), goals (B,4,2), scene (B,6,4)."""
+    rng = np.random.Generator(np.random.PCG64(seed))
+    q0 = np.broadcast_to(POINT_STARTS, (B, 4, 3)).copy()
+    goals = np.broadcast_to(POINT_GOALS, (B, 4, 2)).copy()
+    if jitter > 0:
+        todo = np.arange(B)
+        while len(todo):
+            n = len(todo)
+            q = np.broadcast_to(POINT_STARTS, (n, 4, 3)).copy()
+            q[:, :, 0:2] += rng.uniform(-jitter, jitter, (n, 4, 2))
+            g = POINT_GOALS + rng.uniform(-jitter, jitter, (n, 4, 2))
+            ok = point_start_clearance(q) > 0
+            q0[todo[ok]], goals[todo[ok]] = q[ok], g[ok]
+            todo = todo[~ok]
+    scene = np.zeros((B, len(POINT_SCENE), 4))
+    scene[:, :, 0:3] = POINT_SCENE
+    scene[:, :, 3] = POINT_SCENE_RADIUS
+    return q0, goals, scene
+
+
+def point_start_clearance(q0: np.ndarray, radius: float = POINT_RADIUS) -> np.ndarray:
+    """min over robot pairs of the x-y clearance and over robots and scene spheres of the leaf clearance, per scenario."""
+    p = q0[:, :, 0:2]
+    d = np.linalg.norm(p[:, :, None, :] - p[:, None, :, :], axis=-1) - 2 * radius
+    n = q0.shape[1]
+    d[:, np.arange(n), np.arange(n)] = np.inf
+    x = np.concatenate([p, np.full(p.shape[:2] + (1,), 0.05)], axis=-1)
+    ds = np.linalg.norm(x[:, :, None, :] - POINT_SCENE[None, None], axis=-1) - (POINT_SCENE_RADIUS + radius)
+    return np.minimum(d.min(axis=(1, 2)), ds.min(axis=(1, 2)))
+
+
+def point_masses_reach(B: int, seed: int = 0, jitter: float = 0.3, offset: float = 0.5, margin: float = 0.1):
+    """A solvable variant of the point-mass examples: the starts and scene of point_masses(B, seed, jitter), but every
+    robot's goal lies `offset` from its own start in a uniformly drawn direction (PCG64(seed + 1)).  A direction is redrawn
+    while the goal is closer than `margin` to contact with a scene sphere or another robot's goal.  (The examples' own swap
+    goals put two robots' goals inside scene spheres, so no episode of them can succeed.)
+    -> q0 (B,4,3), goals (B,4,2), scene (B,6,4)."""
+    q0, _, scene = point_masses(B, seed, jitter)
+    rng = np.random.Generator(np.random.PCG64(seed + 1))
+    goals = np.zeros((B, 4, 2))
+    todo = np.arange(B)
+    while len(todo):
+        ph = rng.uniform(0.0, 2.0 * math.pi, (len(todo), 4))
+        g = q0[todo, :, 0:2] + offset * np.stack([np.cos(ph), np.sin(ph)], axis=-1)
+        gq = np.concatenate([g, np.zeros(g.shape[:2] + (1,))], axis=-1)
+        ok = point_start_clearance(gq) > margin
+        goals[todo[ok]] = g[ok]
+        todo = todo[~ok]
+    return q0, goals, scene
