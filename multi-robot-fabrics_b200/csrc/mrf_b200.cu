@@ -671,36 +671,40 @@ __global__ void __launch_bounds__(kActThreads)
 }
 
 // ------------------------------------------------------------------------------------------------
-// AoS <-> SoA staging:  aos[b][f] <-> soa[f][b], tiled through shared memory so both sides coalesce
+// Staging layout of the host-pointer entries: host [B][A][F] (array of records) <-> device [F][A][B] (the kernels'
+// structure of arrays).  The host side is a [B][A*F] matrix with column j = a*F + f, the device side holds that column
+// in row f*A + a; tiled through shared memory so that both sides coalesce.  A = 1 is the plain transpose.
 // ------------------------------------------------------------------------------------------------
-template <typename T, bool TO_SOA>
-__global__ void transpose_kernel(const T* __restrict__ in, T* __restrict__ out, long long B, int F) {
+template <typename T, bool TO_DEVICE>
+__global__ void layout_kernel(const T* __restrict__ in, T* __restrict__ out, long long B, int A, int F) {
     __shared__ T tile[32][33];
+    const int AF = A * F;
     const long long b0 = (long long)blockIdx.x * 32;
-    const int f0 = blockIdx.y * 32;
-    if (TO_SOA) {
-        for (int i = threadIdx.y; i < 32; i += blockDim.y) { // rows = b, cols = f (contiguous in aos)
+    const int j0 = blockIdx.y * 32;
+    auto row = [&](int j) { return (long long)(j % F) * A + j / F; }; // device row of host column j
+    if (TO_DEVICE) {
+        for (int i = threadIdx.y; i < 32; i += blockDim.y) { // rows = b, cols = j (contiguous on the host side)
             long long b = b0 + i;
-            int f = f0 + threadIdx.x;
-            if (b < B && f < F) tile[i][threadIdx.x] = in[b * F + f];
+            int j = j0 + threadIdx.x;
+            if (b < B && j < AF) tile[i][threadIdx.x] = in[b * AF + j];
         }
         __syncthreads();
         for (int i = threadIdx.y; i < 32; i += blockDim.y) {
-            int f = f0 + i;
+            int j = j0 + i;
             long long b = b0 + threadIdx.x;
-            if (b < B && f < F) out[(long long)f * B + b] = tile[threadIdx.x][i];
+            if (b < B && j < AF) out[row(j) * B + b] = tile[threadIdx.x][i];
         }
     } else {
-        for (int i = threadIdx.y; i < 32; i += blockDim.y) { // rows = f, cols = b (contiguous in soa)
-            int f = f0 + i;
+        for (int i = threadIdx.y; i < 32; i += blockDim.y) { // rows = j, cols = b (contiguous on the device side)
+            int j = j0 + i;
             long long b = b0 + threadIdx.x;
-            if (b < B && f < F) tile[i][threadIdx.x] = in[(long long)f * B + b];
+            if (b < B && j < AF) tile[i][threadIdx.x] = in[row(j) * B + b];
         }
         __syncthreads();
         for (int i = threadIdx.y; i < 32; i += blockDim.y) {
             long long b = b0 + i;
-            int f = f0 + threadIdx.x;
-            if (b < B && f < F) out[b * F + f] = tile[threadIdx.x][i];
+            int j = j0 + threadIdx.x;
+            if (b < B && j < AF) out[b * AF + j] = tile[threadIdx.x][i];
         }
     }
 }
@@ -1111,26 +1115,6 @@ template <typename T> __global__ void __launch_bounds__(256) fma_peak_kernel(T* 
     out[(size_t)blockIdx.x * blockDim.x + threadIdx.x] = ((a0 + a1) + (a2 + a3)) + ((a4 + a5) + (a6 + a7));
 }
 
-// AoS records [B][Ro][Fi] -> SoA [Fi][Ro][B] in one pass (the layout the kernels read), same 32x33 tiling
-template <typename T>
-__global__ void records_to_soa_kernel(const T* __restrict__ in, T* __restrict__ out, long long B, int Ro, int Fi) {
-    __shared__ T tile[32][33];
-    const int F = Ro * Fi;
-    const long long b0 = (long long)blockIdx.x * 32;
-    const int f0 = blockIdx.y * 32;
-    for (int i = threadIdx.y; i < 32; i += blockDim.y) {
-        long long b = b0 + i;
-        int f = f0 + threadIdx.x;
-        if (b < B && f < F) tile[i][threadIdx.x] = in[b * F + f];
-    }
-    __syncthreads();
-    for (int i = threadIdx.y; i < 32; i += blockDim.y) {
-        int f = f0 + i; // input column = r * Fi + field
-        long long b = b0 + threadIdx.x;
-        if (b < B && f < F) out[((long long)(f % Fi) * Ro + f / Fi) * B + b] = tile[threadIdx.x][i];
-    }
-}
-
 } // namespace mrf
 
 // =================================================================================================
@@ -1157,8 +1141,9 @@ struct MrfHandle_ {
     DevCfg<double> c64;
     cudaStream_t stream, s_copy, s_chunk[8];
     cudaEvent_t ev0, ev1, ev_up[8], ev_free, ev_chunk[8];
-    void* stage[8];
-    size_t stage_bytes[8];
+    // device scratch of the synchronous host entries (scratch_reset / scratch_take): blocks, the last one being filled
+    std::vector<void*> scratch;
+    size_t scratch_cap, scratch_off, scratch_used; // size and fill of the last block, bytes taken by the current call
     long long launches;
     double last_ms;
     long long coop_max_batch; // batches up to this size use the cooperative low-latency rollout kernel
@@ -1335,8 +1320,7 @@ extern "C" int mrf_create(const MrfConfig* cfg, int device, mrf_handle_t* out) {
 extern "C" int mrf_destroy(mrf_handle_t h) {
     if (!h) return MRF_OK;
     cudaSetDevice(h->device);
-    for (int i = 0; i < 8; ++i)
-        if (h->stage[i]) cudaFree(h->stage[i]);
+    for (void* p : h->scratch) cudaFree(p);
     if (h->d_sync) cudaFree(h->d_sync);
     for (int i = 0; i < 4; ++i) {
         if (h->rf_buf[i]) cudaFree(h->rf_buf[i]);
@@ -1799,46 +1783,81 @@ extern "C" int mrf_guard_stats(mrf_handle_t h, int64_t* out) {
 }
 
 // ---------------------------------- host-pointer entries ----------------------------------------
-static int stage_reserve(mrf_handle_t h, int slot, size_t bytes) {
-    if (h->stage_bytes[slot] >= bytes) return MRF_OK;
-    if (h->stage[slot]) MRF_CUDA(cudaFree(h->stage[slot]));
-    h->stage[slot] = nullptr;
-    h->stage_bytes[slot] = 0;
-    size_t want = bytes + bytes / 4;
-    if (cudaMalloc(&h->stage[slot], want) != cudaSuccess) {
+// Device scratch of the synchronous host entries.  Every call starts with scratch_reset and takes a distinct region
+// for each array it stages; no region is reused within a call, so the staging needs no synchronisation of its own.  A
+// call that outgrows the last block continues in a new one and keeps the old (its earlier regions live there).  The
+// next reset frees them all -- cudaFree waits for the device, so no earlier work still reads them -- and allocates one
+// block that holds the whole previous call: repeated calls with the same shapes allocate nothing.
+static int scratch_grow(mrf_handle_t h, size_t bytes) {
+    const size_t want = bytes + bytes / 4;
+    void* p = nullptr;
+    if (cudaMalloc(&p, want) != cudaSuccess) {
         cudaGetLastError();
         return fail(MRF_ENOMEM, "mrf: device allocation failed");
     }
-    h->stage_bytes[slot] = want;
+    h->scratch.push_back(p);
+    h->scratch_cap = want;
+    h->scratch_off = 0;
     return MRF_OK;
 }
 
-// host AoS [B][F] -> device SoA [F][B] in stage[soa_slot] (via stage[aos_slot])
-template <typename T>
-static int upload_soa(mrf_handle_t h, const T* host, long long B, int F, int aos_slot, int soa_slot) {
-    const size_t bytes = sizeof(T) * (size_t)B * F;
-    int rc = stage_reserve(h, aos_slot, bytes);
-    if (rc) return rc;
-    rc = stage_reserve(h, soa_slot, bytes);
-    if (rc) return rc;
-    MRF_CUDA(cudaMemcpyAsync(h->stage[aos_slot], host, bytes, cudaMemcpyHostToDevice, h->stream));
-    dim3 grid((unsigned)((B + 31) / 32), (unsigned)((F + 31) / 32)), block(32, 8);
-    transpose_kernel<T, true><<<grid, block, 0, h->stream>>>((const T*)h->stage[aos_slot], (T*)h->stage[soa_slot], B, F);
+static int scratch_reset(mrf_handle_t h) {
+    const size_t used = h->scratch_used;
+    h->scratch_off = h->scratch_used = 0;
+    if (h->scratch.size() <= 1) return MRF_OK;
+    for (void* p : h->scratch) MRF_CUDA(cudaFree(p));
+    h->scratch.clear();
+    h->scratch_cap = 0;
+    return scratch_grow(h, used);
+}
+
+template <typename T> static int scratch_take(mrf_handle_t h, size_t n, T** out) {
+    const size_t bytes = (sizeof(T) * n + 255) / 256 * 256;
+    if (h->scratch_off + bytes > h->scratch_cap) {
+        int rc = scratch_grow(h, h->scratch_used + bytes);
+        if (rc) return rc;
+    }
+    *out = (T*)((char*)h->scratch.back() + h->scratch_off);
+    h->scratch_off += bytes;
+    h->scratch_used += bytes;
+    return MRF_OK;
+}
+
+template <typename T, bool TO_DEVICE>
+static int launch_layout(mrf_handle_t h, const T* in, T* out, long long B, int A, int F, cudaStream_t stream) {
+    dim3 grid((unsigned)((B + 31) / 32), (unsigned)((A * F + 31) / 32)), block(32, 8);
+    layout_kernel<T, TO_DEVICE><<<grid, block, 0, stream>>>(in, out, B, A, F);
     MRF_CUDA(cudaGetLastError());
     h->launches += 1;
     return MRF_OK;
 }
-// device SoA [F][B] in stage[soa_slot] -> host AoS [B][F] (via stage[aos_slot])
+
+// host [B][A][F] -> device [F][A][B] in scratch: one copy and one layout kernel on h->stream
 template <typename T>
-static int download_aos(mrf_handle_t h, T* host, long long B, int F, int soa_slot, int aos_slot) {
-    const size_t bytes = sizeof(T) * (size_t)B * F;
-    int rc = stage_reserve(h, aos_slot, bytes);
+static int stage_in(mrf_handle_t h, const T* host, long long B, int A, int F, const T** dev) {
+    const size_t n = (size_t)B * A * F;
+    T *raw, *out;
+    int rc = scratch_take(h, n, &raw);
+    if (!rc) rc = scratch_take(h, n, &out);
     if (rc) return rc;
-    dim3 grid((unsigned)((B + 31) / 32), (unsigned)((F + 31) / 32)), block(32, 8);
-    transpose_kernel<T, false><<<grid, block, 0, h->stream>>>((const T*)h->stage[soa_slot], (T*)h->stage[aos_slot], B, F);
-    MRF_CUDA(cudaGetLastError());
-    h->launches += 1;
-    MRF_CUDA(cudaMemcpyAsync(host, h->stage[aos_slot], bytes, cudaMemcpyDeviceToHost, h->stream));
+    MRF_CUDA(cudaMemcpyAsync(raw, host, sizeof(T) * n, cudaMemcpyHostToDevice, h->stream));
+    *dev = out;
+    return launch_layout<T, true>(h, raw, out, B, A, F, h->stream);
+}
+
+// device [F][A][B] -> host [B][A][F] on h->stream; nothing when host is null
+template <typename T>
+static int stage_out(mrf_handle_t h, const T* dev, long long B, int A, int F, T* host) {
+    if (!host) return MRF_OK;
+    const size_t n = (size_t)B * A * F;
+    if (A * F > 1) { // with one field per scenario both layouts are the same array
+        T* tmp;
+        int rc = scratch_take(h, n, &tmp);
+        if (!rc) rc = launch_layout<T, false>(h, dev, tmp, B, A, F, h->stream);
+        if (rc) return rc;
+        dev = tmp;
+    }
+    MRF_CUDA(cudaMemcpyAsync(host, dev, sizeof(T) * n, cudaMemcpyDeviceToHost, h->stream));
     return MRF_OK;
 }
 
@@ -1850,41 +1869,19 @@ static int finish_timed(mrf_handle_t h) {
     return MRF_OK;
 }
 
-// The host AoS order [B][R][F] is, per scenario, R records back to back: as a [B][R*F] matrix its transpose is
-// [R*F][B] = [r][f][b]; the kernels want [f][r][b].  The kernels' loader takes (f, r) -> row, so for the host
-// path the records are uploaded one robot at a time into the [f][r][b] layout.
-template <typename T>
-static int upload_records(mrf_handle_t h, const T* rec, long long B, int R, int slot_aos, int slot_tmp, int slot_soa) {
-    // upload whole AoS once, transpose to [R*F][B] (= [r][f][b]), then permute rows to [f][r][b] with 2-D copies
-    int rc = upload_soa<T>(h, rec, B, R * MRF_REC, slot_aos, slot_tmp);
-    if (rc) return rc;
-    if (R == 1) return MRF_OK; // [f][b] already
-    rc = stage_reserve(h, slot_soa, sizeof(T) * (size_t)B * R * MRF_REC);
-    if (rc) return rc;
-    for (int r = 0; r < R; ++r) // rows r*F+f  ->  rows f*R+r : strided 2-D copy per robot
-        MRF_CUDA(cudaMemcpy2DAsync((T*)h->stage[slot_soa] + (size_t)r * B, sizeof(T) * (size_t)R * B,
-                                   (const T*)h->stage[slot_tmp] + (size_t)r * MRF_REC * B, sizeof(T) * (size_t)B,
-                                   sizeof(T) * (size_t)B, MRF_REC, cudaMemcpyDeviceToDevice, h->stream));
-    return MRF_OK;
-}
-
 // Large batches without trajectory output: the batch is cut into chunks; the H2D copy of chunk c+1 (copy stream)
-// overlaps the transpose + rollout + result read-back of chunk c (compute stream).
+// overlaps the layout kernels + rollout + result read-back of chunk c (compute stream).
 template <typename T>
 static int rollout_host_pipelined(mrf_handle_t h, const T* rec, int N, T* avg_vel, T* x_ee, T* goal_est, int64_t B) {
     const int R = h->cfg.n_robots, C = B >= 32768 ? 8 : 4;
     const long long Bc = (((B + C - 1) / C) + 31) / 32 * 32; // chunk size, multiple of the CTA tile
-    const size_t rec_elems = (size_t)B * R * MRF_REC;
-    int rc = stage_reserve(h, 0, sizeof(T) * rec_elems);   // AoS records
-    if (rc) return rc;
-    rc = stage_reserve(h, 2, sizeof(T) * (size_t)Bc * C * R * MRF_REC); // SoA records, one block per chunk
-    if (rc) return rc;
     const size_t per = (size_t)(R + 3 * R + 3);
-    rc = stage_reserve(h, 3, sizeof(T) * per * Bc * C);   // SoA results per chunk
+    T *d_aos, *d_soa, *d_res, *a_avg;
+    int rc = scratch_take(h, (size_t)B * R * MRF_REC, &d_aos);               // records as uploaded
+    if (!rc) rc = scratch_take(h, (size_t)Bc * C * R * MRF_REC, &d_soa);     // device layout, one block per chunk
+    if (!rc) rc = scratch_take(h, per * Bc * C, &d_res);                     // device-layout results per chunk
+    if (!rc) rc = scratch_take(h, per * B, &a_avg);                          // host order: avg [B][R], x_ee [B][3R], goal [B][3]
     if (rc) return rc;
-    rc = stage_reserve(h, 5, sizeof(T) * per * B);        // AoS results: avg [B][R], x_ee [B][3R], goal [B][3]
-    if (rc) return rc;
-    T* a_avg = (T*)h->stage[5];
     T* a_xee = a_avg + (size_t)B * R;
     T* a_goal = a_xee + (size_t)B * 3 * R;
     // make sure earlier work on the compute stream no longer reads the staging buffers the copy stream overwrites
@@ -1900,30 +1897,26 @@ static int rollout_host_pipelined(mrf_handle_t h, const T* rec, int N, T* avg_ve
         // alone is less than one wave of CTAs), only the copy -> compute order of each chunk is enforced
         cudaStream_t cs = h->s_chunk[c];
         MRF_CUDA(cudaStreamWaitEvent(cs, h->ev_free, 0));
-        T* d_aos = (T*)h->stage[0] + (size_t)lo * R * MRF_REC;
-        MRF_CUDA(cudaMemcpyAsync(d_aos, rec + (size_t)lo * R * MRF_REC, sizeof(T) * (size_t)n * R * MRF_REC,
+        T* c_aos = d_aos + (size_t)lo * R * MRF_REC;
+        MRF_CUDA(cudaMemcpyAsync(c_aos, rec + (size_t)lo * R * MRF_REC, sizeof(T) * (size_t)n * R * MRF_REC,
                                  cudaMemcpyHostToDevice, h->s_copy));
         MRF_CUDA(cudaEventRecord(h->ev_up[c], h->s_copy));
         MRF_CUDA(cudaStreamWaitEvent(cs, h->ev_up[c], 0));
-        T* d_soa = (T*)h->stage[2] + (size_t)c * Bc * R * MRF_REC;
-        dim3 grid((unsigned)((n + 31) / 32), (unsigned)((R * MRF_REC + 31) / 32)), block(32, 8);
-        records_to_soa_kernel<T><<<grid, block, 0, cs>>>(d_aos, d_soa, n, R, MRF_REC);
-        MRF_CUDA(cudaGetLastError());
-        h->launches += 1;
-        T* d_avg = (T*)h->stage[3] + (size_t)c * Bc * per;
+        T* c_soa = d_soa + (size_t)c * Bc * R * MRF_REC;
+        rc = launch_layout<T, true>(h, c_aos, c_soa, n, R, MRF_REC, cs);
+        if (rc) return rc;
+        T* d_avg = d_res + (size_t)c * Bc * per;
         T* d_xee = d_avg + (size_t)R * n;
         T* d_goal = d_xee + (size_t)3 * R * n;
-        rc = rollout_dev<T>(h, d_soa, N, d_avg, d_xee, d_goal, nullptr, nullptr, n, cs);
+        rc = rollout_dev<T>(h, c_soa, N, d_avg, d_xee, d_goal, nullptr, nullptr, n, cs);
         if (rc) return rc;
         struct { T* src; T* dst; T* host; int F; } outs[3] = {{d_avg, a_avg + (size_t)lo * R, avg_vel, R},
                                                               {d_xee, a_xee + (size_t)lo * 3 * R, x_ee, 3 * R},
                                                               {d_goal, a_goal + (size_t)lo * 3, goal_est, 3}};
         for (auto& o : outs) {
             if (!o.host) continue;
-            dim3 g2((unsigned)((n + 31) / 32), (unsigned)((o.F + 31) / 32));
-            transpose_kernel<T, false><<<g2, block, 0, cs>>>(o.src, o.dst, n, o.F);
-            MRF_CUDA(cudaGetLastError());
-            h->launches += 1;
+            rc = launch_layout<T, false>(h, o.src, o.dst, n, 1, o.F, cs);
+            if (rc) return rc;
             MRF_CUDA(cudaMemcpyAsync(o.host + (size_t)lo * o.F, o.dst, sizeof(T) * (size_t)n * o.F, cudaMemcpyDeviceToHost, cs));
         }
         MRF_CUDA(cudaEventRecord(h->ev_chunk[c], cs));
@@ -1947,7 +1940,7 @@ static void* pinned_view(const void* p) {
 
 // Page-locked records: ONE kernel launch reads the caller's records straight from host memory (record order, coalesced
 // 16-byte loads per tile) and writes avg / x_ee / goal straight back -- the CTA scheduler overlaps the PCIe reads of
-// later tiles with the horizons of earlier ones, so there is no staging copy, no transpose and no chunk pipeline.
+// later tiles with the horizons of earlier ones, so there is no staging copy, no layout kernel and no chunk pipeline.
 // Results whose host buffer is not page-locked go through a device buffer and one copy.
 template <typename T>
 static int rollout_host_zerocopy(mrf_handle_t h, const T* rec_view, int N, T* avg_vel, T* x_ee, T* goal_est, int64_t B) {
@@ -1955,19 +1948,14 @@ static int rollout_host_zerocopy(mrf_handle_t h, const T* rec_view, int N, T* av
     struct Out { T* host; T* dev; size_t n; bool direct; } outs[3] = {{avg_vel, nullptr, (size_t)B * R, false},
                                                                       {x_ee, nullptr, (size_t)B * 3 * R, false},
                                                                       {goal_est, nullptr, (size_t)B * 3, false}};
-    size_t staged = 0;
     for (auto& o : outs) {
         if (!o.host) continue;
         o.dev = (T*)pinned_view(o.host);
         o.direct = o.dev != nullptr;
-        if (!o.direct) staged += o.n;
-    }
-    if (staged) {
-        int rc = stage_reserve(h, 5, sizeof(T) * staged);
-        if (rc) return rc;
-        T* p = (T*)h->stage[5];
-        for (auto& o : outs)
-            if (o.host && !o.direct) { o.dev = p; p += o.n; }
+        if (!o.direct) {
+            int rc = scratch_take(h, o.n, &o.dev);
+            if (rc) return rc;
+        }
     }
     MRF_CUDA(cudaEventRecord(h->ev0, h->stream));
     int rc = rollout_dev<T>(h, rec_view, N, outs[0].dev, outs[1].dev, outs[2].dev, nullptr, nullptr, B, h->stream, true);
@@ -1985,73 +1973,33 @@ static int rollout_host(mrf_handle_t h, const T* rec, int N, T* avg_vel, T* x_ee
     if (B <= 0 || N <= 0) return fail(MRF_EINVAL, "mrf_rollout_host: B and N must be positive");
     MRF_CUDA(cudaSetDevice(h->device));
     const int R = h->cfg.n_robots;
+    int rc = scratch_reset(h);
+    if (rc) return rc;
     if (!qN && !qdN && B >= 8192) {
         if (h->zero_copy)
             if (const T* view = (const T*)pinned_view(rec)) return rollout_host_zerocopy<T>(h, view, N, avg_vel, x_ee, goal_est, B);
         return rollout_host_pipelined<T>(h, rec, N, avg_vel, x_ee, goal_est, B);
     }
-    int rc = upload_records<T>(h, rec, B, R, 0, 1, 2);
-    if (rc) return rc;
-    const T* d_rec = (const T*)h->stage[R == 1 ? 1 : 2];
-    // outputs (SoA) packed in stage[3]: avg[R][B], x_ee[R][3][B], goal[3][B], then optional trajectories in stage[4]
-    const size_t n_small = (size_t)B * (R + 3 * R + 3);
-    rc = stage_reserve(h, 3, sizeof(T) * n_small);
-    if (rc) return rc;
-    T* d_avg = (T*)h->stage[3];
-    T* d_xee = d_avg + (size_t)R * B;
-    T* d_goal = d_xee + (size_t)3 * R * B;
-    T *d_q = nullptr, *d_qd = nullptr;
+    const T* d_rec;
+    T *d_avg, *d_xee, *d_goal, *d_q = nullptr, *d_qd = nullptr;
     const size_t n_traj = (size_t)B * R * N * MRF_DOF;
-    if (qN || qdN) {
-        rc = stage_reserve(h, 4, sizeof(T) * n_traj * 2);
-        if (rc) return rc;
-        if (qN) d_q = (T*)h->stage[4];
-        if (qdN) d_qd = (T*)h->stage[4] + n_traj;
-    }
+    rc = stage_in(h, rec, B, R, MRF_REC, &d_rec);
+    if (!rc) rc = scratch_take(h, (size_t)B * R, &d_avg);          // [R][B]
+    if (!rc) rc = scratch_take(h, (size_t)B * 3 * R, &d_xee);      // [R][3][B]
+    if (!rc) rc = scratch_take(h, (size_t)B * 3, &d_goal);         // [3][B]
+    if (!rc && qN) rc = scratch_take(h, n_traj, &d_q);             // [R][N][7][B]
+    if (!rc && qdN) rc = scratch_take(h, n_traj, &d_qd);
+    if (rc) return rc;
     MRF_CUDA(cudaEventRecord(h->ev0, h->stream));
     rc = rollout_dev<T>(h, d_rec, N, d_avg, d_xee, d_goal, d_q, d_qd, B, h->stream);
     if (rc) return rc;
     MRF_CUDA(cudaEventRecord(h->ev1, h->stream));
-    // SoA [R][B] -> AoS [B][R] etc.
-    if (avg_vel) { rc = download_aos<T>(h, avg_vel, B, R, 3, 5); if (rc) return rc; }
-    if (x_ee) {
-        // d_xee is [R*3][B]
-        const size_t bytes = sizeof(T) * (size_t)B * 3 * R;
-        rc = stage_reserve(h, 6, bytes);
-        if (rc) return rc;
-        dim3 grid((unsigned)((B + 31) / 32), (unsigned)((3 * R + 31) / 32)), block(32, 8);
-        transpose_kernel<T, false><<<grid, block, 0, h->stream>>>(d_xee, (T*)h->stage[6], B, 3 * R);
-        MRF_CUDA(cudaGetLastError());
-        h->launches += 1;
-        MRF_CUDA(cudaMemcpyAsync(x_ee, h->stage[6], bytes, cudaMemcpyDeviceToHost, h->stream));
-    }
-    if (goal_est) {
-        const size_t bytes = sizeof(T) * (size_t)B * 3;
-        rc = stage_reserve(h, 7, bytes);
-        if (rc) return rc;
-        dim3 grid((unsigned)((B + 31) / 32), 1), block(32, 8);
-        transpose_kernel<T, false><<<grid, block, 0, h->stream>>>(d_goal, (T*)h->stage[7], B, 3);
-        MRF_CUDA(cudaGetLastError());
-        h->launches += 1;
-        MRF_CUDA(cudaMemcpyAsync(goal_est, h->stage[7], bytes, cudaMemcpyDeviceToHost, h->stream));
-    }
-    if (qN || qdN) {
-        // device [R][N][7][B] -> host [B][R][N][7]: one transpose of a [R*N*7][B] matrix
-        const int F = R * N * MRF_DOF;
-        rc = stage_reserve(h, 0, sizeof(T) * n_traj); // the AoS record staging is free again
-        if (rc) return rc;
-        dim3 grid((unsigned)((B + 31) / 32), (unsigned)((F + 31) / 32)), block(32, 8);
-        for (int which = 0; which < 2; ++which) {
-            T* hostp = which ? qdN : qN;
-            T* devp = which ? d_qd : d_q;
-            if (!hostp) continue;
-            transpose_kernel<T, false><<<grid, block, 0, h->stream>>>(devp, (T*)h->stage[0], B, F);
-            MRF_CUDA(cudaGetLastError());
-            h->launches += 1;
-            MRF_CUDA(cudaMemcpyAsync(hostp, h->stage[0], sizeof(T) * n_traj, cudaMemcpyDeviceToHost, h->stream));
-            MRF_CUDA(cudaStreamSynchronize(h->stream));
-        }
-    }
+    rc = stage_out(h, d_avg, B, 1, R, avg_vel);
+    if (!rc) rc = stage_out(h, d_xee, B, 1, 3 * R, x_ee);
+    if (!rc) rc = stage_out(h, d_goal, B, 1, 3, goal_est);
+    if (!rc) rc = stage_out(h, d_q, B, 1, R * N * MRF_DOF, qN);
+    if (!rc) rc = stage_out(h, d_qd, B, 1, R * N * MRF_DOF, qdN);
+    if (rc) return rc;
     return finish_timed(h);
 }
 
@@ -2263,74 +2211,28 @@ static int action_host(mrf_handle_t h, int robot_first, int n_rob, const T* rec,
     if (B <= 0 || S < 0 || n_rob < 1) return fail(MRF_EINVAL, "mrf_action_host: bad sizes");
     MRF_CUDA(cudaSetDevice(h->device));
     const int R = n_rob;
-    int rc = upload_records<T>(h, rec, B, R, 0, 1, 2);
-    if (rc) return rc;
-    const T* d_rec = (const T*)h->stage[R == 1 ? 1 : 2];
-    const T* d_obst = nullptr;
-    if (S > 0) {
-        // host [B][R][S][10] -> [R*S*10][B] = [r][o][c][b]; kernels want [o][c][r][b]
-        rc = upload_soa<T>(h, obst, B, R * S * MRF_OBST, 3, 4);
-        if (rc) return rc;
-        if (R == 1) {
-            d_obst = (const T*)h->stage[4];
-        } else {
-            rc = stage_reserve(h, 5, sizeof(T) * (size_t)B * R * S * MRF_OBST);
-            if (rc) return rc;
-            for (int r = 0; r < R; ++r)
-                MRF_CUDA(cudaMemcpy2DAsync((T*)h->stage[5] + (size_t)r * B, sizeof(T) * (size_t)R * B,
-                                           (const T*)h->stage[4] + (size_t)r * S * MRF_OBST * B, sizeof(T) * (size_t)B,
-                                           sizeof(T) * (size_t)B, (size_t)S * MRF_OBST, cudaMemcpyDeviceToDevice,
-                                           h->stream));
-            d_obst = (const T*)h->stage[5];
-        }
-    }
-    const int Fo = CART ? 1 : MRF_DOF * R;
-    rc = stage_reserve(h, 6, sizeof(T) * (size_t)B * Fo);
-    if (rc) return rc;
-    T *d_q = nullptr, *d_qd = nullptr;
+    const T *d_rec, *d_obst = nullptr;
+    T *d_out, *d_q = nullptr, *d_qd = nullptr;
     const size_t n_traj = CART ? (size_t)B * N * MRF_DOF : 0;
-    if (CART && (qN || qdN)) {
-        rc = stage_reserve(h, 7, sizeof(T) * n_traj * 2);
-        if (rc) return rc;
-        if (qN) d_q = (T*)h->stage[7];
-        if (qdN) d_qd = (T*)h->stage[7] + n_traj;
-    }
+    int rc = scratch_reset(h);
+    if (!rc) rc = stage_in(h, rec, B, R, MRF_REC, &d_rec);
+    if (!rc && S > 0) rc = stage_in(h, obst, B, R, S * MRF_OBST, &d_obst);          // [S][10][R][B]
+    if (!rc) rc = scratch_take(h, (size_t)B * (CART ? 1 : MRF_DOF * R), &d_out);    // avg_vel [B] or action [7][R][B]
+    if (!rc && CART && qN) rc = scratch_take(h, n_traj, &d_q);                      // [N][7][B]
+    if (!rc && CART && qdN) rc = scratch_take(h, n_traj, &d_qd);
+    if (rc) return rc;
     MRF_CUDA(cudaEventRecord(h->ev0, h->stream));
-    rc = action_dev<T, CART>(h, robot_first, n_rob, d_rec, S, d_obst, N, (T*)h->stage[6], d_q, d_qd, B, h->stream);
+    rc = action_dev<T, CART>(h, robot_first, n_rob, d_rec, S, d_obst, N, d_out, d_q, d_qd, B, h->stream);
     if (rc) return rc;
     MRF_CUDA(cudaEventRecord(h->ev1, h->stream));
     if (CART) {
-        if (out) MRF_CUDA(cudaMemcpyAsync(out, h->stage[6], sizeof(T) * (size_t)B, cudaMemcpyDeviceToHost, h->stream));
-        const int F = N * MRF_DOF;
-        dim3 grid((unsigned)((B + 31) / 32), (unsigned)((F + 31) / 32)), block(32, 8);
-        for (int which = 0; which < 2; ++which) {
-            T* hostp = which ? qdN : qN;
-            T* devp = which ? d_qd : d_q;
-            if (!hostp) continue;
-            rc = stage_reserve(h, 0, sizeof(T) * n_traj);
-            if (rc) return rc;
-            transpose_kernel<T, false><<<grid, block, 0, h->stream>>>(devp, (T*)h->stage[0], B, F);
-            MRF_CUDA(cudaGetLastError());
-            h->launches += 1;
-            MRF_CUDA(cudaMemcpyAsync(hostp, h->stage[0], sizeof(T) * n_traj, cudaMemcpyDeviceToHost, h->stream));
-            MRF_CUDA(cudaStreamSynchronize(h->stream));
-        }
+        rc = stage_out(h, d_out, B, 1, 1, out);
+        if (!rc) rc = stage_out(h, d_q, B, 1, N * MRF_DOF, qN);
+        if (!rc) rc = stage_out(h, d_qd, B, 1, N * MRF_DOF, qdN);
     } else {
-        // device [7][R][B] -> host [B][R][7]: permute rows to [R][7][B] first
-        if (R == 1) {
-            rc = download_aos<T>(h, out, B, MRF_DOF, 6, 0);
-            if (rc) return rc;
-        } else {
-            rc = stage_reserve(h, 7, sizeof(T) * (size_t)B * Fo);
-            if (rc) return rc;
-            for (int r = 0; r < R; ++r)
-                MRF_CUDA(cudaMemcpy2DAsync((T*)h->stage[7] + (size_t)r * MRF_DOF * B, sizeof(T) * (size_t)B,
-                                           (const T*)h->stage[6] + (size_t)r * B, sizeof(T) * (size_t)R * B,
-                                           sizeof(T) * (size_t)B, MRF_DOF, cudaMemcpyDeviceToDevice, h->stream));
-            rc = download_aos<T>(h, out, B, MRF_DOF * R, 7, 0);
-            if (rc) return rc;
-        }
+        rc = stage_out(h, d_out, B, R, MRF_DOF, out);
     }
+    if (rc) return rc;
     return finish_timed(h);
 }
 
@@ -2364,45 +2266,24 @@ extern "C" int mrf_kinematics_host_f64(mrf_handle_t h, const double* q, const do
     if (!h || !q || !qdot) return fail(MRF_EINVAL, "mrf_kinematics_host: null argument");
     if (B <= 0) return fail(MRF_EINVAL, "mrf_kinematics_host: B must be positive");
     MRF_CUDA(cudaSetDevice(h->device));
-    const int R = h->cfg.n_robots;
-    // host [B][R][7] -> [R*7][B] = [r][i][b]; kernel wants [i][r][b]
-    const double* src[2] = {q, qdot};
-    for (int w = 0; w < 2; ++w) {
-        int rc = upload_soa<double>(h, src[w], B, R * MRF_DOF, 0, 1);
-        if (rc) return rc;
-        rc = stage_reserve(h, 2 + w, sizeof(double) * (size_t)B * R * MRF_DOF);
-        if (rc) return rc;
-        for (int r = 0; r < R; ++r)
-            MRF_CUDA(cudaMemcpy2DAsync((double*)h->stage[2 + w] + (size_t)r * B, sizeof(double) * (size_t)R * B,
-                                       (const double*)h->stage[1] + (size_t)r * MRF_DOF * B, sizeof(double) * (size_t)B,
-                                       sizeof(double) * (size_t)B, MRF_DOF, cudaMemcpyDeviceToDevice, h->stream));
-        MRF_CUDA(cudaStreamSynchronize(h->stream));
-    }
-    const size_t n_out = (size_t)B * R * MRF_NLINKS * 3;
-    int rc = stage_reserve(h, 4, sizeof(double) * n_out * 3);
+    const int R = h->cfg.n_robots, F = MRF_NLINKS * 3; // outputs: device [l][c][r][b], host [b][r][l][c]
+    const double *d_q, *d_qd;
+    double *d_x, *d_v, *d_a;
+    int rc = scratch_reset(h);
+    if (!rc) rc = stage_in(h, q, B, R, MRF_DOF, &d_q);
+    if (!rc) rc = stage_in(h, qdot, B, R, MRF_DOF, &d_qd);
+    if (!rc) rc = scratch_take(h, (size_t)B * R * F, &d_x);
+    if (!rc) rc = scratch_take(h, (size_t)B * R * F, &d_v);
+    if (!rc) rc = scratch_take(h, (size_t)B * R * F, &d_a);
     if (rc) return rc;
-    double* d_x = (double*)h->stage[4];
-    double* d_v = d_x + n_out;
-    double* d_a = d_v + n_out;
     MRF_CUDA(cudaEventRecord(h->ev0, h->stream));
-    rc = kinematics_dev<double>(h, (const double*)h->stage[2], (const double*)h->stage[3], d_x, d_v, d_a, B, h->stream);
+    rc = kinematics_dev<double>(h, d_q, d_qd, d_x, d_v, d_a, B, h->stream);
     if (rc) return rc;
     MRF_CUDA(cudaEventRecord(h->ev1, h->stream));
-    // device [l][c][r][b] -> host [b][r][l][c]
-    double* outs[3] = {x, v, a};
-    double* devs[3] = {d_x, d_v, d_a};
-    rc = stage_reserve(h, 5, sizeof(double) * n_out);
+    rc = stage_out(h, d_x, B, R, F, x);
+    if (!rc) rc = stage_out(h, d_v, B, R, F, v);
+    if (!rc) rc = stage_out(h, d_a, B, R, F, a);
     if (rc) return rc;
-    for (int w = 0; w < 3; ++w) {
-        if (!outs[w]) continue;
-        for (int r = 0; r < R; ++r) // rows (l*3+c)*R + r -> rows r*24 + (l*3+c)
-            MRF_CUDA(cudaMemcpy2DAsync((double*)h->stage[5] + (size_t)r * 24 * B, sizeof(double) * (size_t)B,
-                                       devs[w] + (size_t)r * B, sizeof(double) * (size_t)R * B, sizeof(double) * (size_t)B,
-                                       24, cudaMemcpyDeviceToDevice, h->stream));
-        rc = download_aos<double>(h, outs[w], B, R * 24, 5, 0);
-        if (rc) return rc;
-        MRF_CUDA(cudaStreamSynchronize(h->stream));
-    }
     return finish_timed(h);
 }
 
@@ -2445,12 +2326,12 @@ extern "C" int mrf_deadlock_host_f64(mrf_handle_t h, const double* x_ee, double*
         for (int k = 0; k < 4; ++k) qi[(size_t)k * B + b] = st_int[b * 4 + k];
         for (int k = 0; k < 3; ++k) ps[(size_t)k * B + b] = st_goal[b * 3 + k];
     }
-    int rc = stage_reserve(h, 0, sizeof(double) * nd);
+    double* dd;
+    int32_t* di;
+    int rc = scratch_reset(h);
+    if (!rc) rc = scratch_take(h, nd, &dd);
+    if (!rc) rc = scratch_take(h, ni, &di);
     if (rc) return rc;
-    rc = stage_reserve(h, 1, sizeof(int32_t) * ni);
-    if (rc) return rc;
-    double* dd = (double*)h->stage[0];
-    int32_t* di = (int32_t*)h->stage[1];
     MRF_CUDA(cudaMemcpyAsync(dd, hd.data(), sizeof(double) * nd, cudaMemcpyHostToDevice, h->stream));
     MRF_CUDA(cudaMemcpyAsync(di, hi.data(), sizeof(int32_t) * ni, cudaMemcpyHostToDevice, h->stream));
     MRF_CUDA(cudaEventRecord(h->ev0, h->stream));
@@ -2533,18 +2414,19 @@ extern "C" int mrf_point_action_host_f64(mrf_handle_t h, const double* rec, int 
     if (!h || !rec || !action || (Ss > 0 && !stat) || (Sd > 0 && !dyn)) return fail(MRF_EINVAL, "mrf_point_action_host: null argument");
     if (B <= 0) return fail(MRF_EINVAL, "mrf_point_action_host: B must be positive");
     MRF_CUDA(cudaSetDevice(h->device));
-    int rc = upload_soa<double>(h, rec, B, 10, 0, 1);
-    if (rc) return rc;
-    if (Ss > 0) { rc = upload_soa<double>(h, stat, B, Ss * 4, 2, 3); if (rc) return rc; }
-    if (Sd > 0) { rc = upload_soa<double>(h, dyn, B, Sd * 7, 4, 5); if (rc) return rc; }
-    rc = stage_reserve(h, 6, sizeof(double) * (size_t)B * 3);
+    const double *d_rec, *d_stat = nullptr, *d_dyn = nullptr;
+    double* d_act;
+    int rc = scratch_reset(h);
+    if (!rc) rc = stage_in(h, rec, B, 1, 10, &d_rec);
+    if (!rc && Ss > 0) rc = stage_in(h, stat, B, 1, Ss * 4, &d_stat);
+    if (!rc && Sd > 0) rc = stage_in(h, dyn, B, 1, Sd * 7, &d_dyn);
+    if (!rc) rc = scratch_take(h, (size_t)B * 3, &d_act);
     if (rc) return rc;
     MRF_CUDA(cudaEventRecord(h->ev0, h->stream));
-    rc = point_action_dev<double>(h, (const double*)h->stage[1], Ss, (const double*)h->stage[3], Sd,
-                                  (const double*)h->stage[5], (double*)h->stage[6], B, h->stream);
+    rc = point_action_dev<double>(h, d_rec, Ss, d_stat, Sd, d_dyn, d_act, B, h->stream);
     if (rc) return rc;
     MRF_CUDA(cudaEventRecord(h->ev1, h->stream));
-    rc = download_aos<double>(h, action, B, 3, 6, 7);
+    rc = stage_out(h, d_act, B, 1, 3, action);
     if (rc) return rc;
     return finish_timed(h);
 }
@@ -2895,12 +2777,14 @@ template <typename T> static int fma_peak(mrf_handle_t h, double* tflops) {
     cudaDeviceProp prop;
     MRF_CUDA(cudaGetDeviceProperties(&prop, h->device));
     const int blocks = prop.multiProcessorCount * 8, threads = 256, iters = 1 << 15;
-    int rc = stage_reserve(h, 0, sizeof(T) * (size_t)blocks * threads);
+    T* out;
+    int rc = scratch_reset(h);
+    if (!rc) rc = scratch_take(h, (size_t)blocks * threads, &out);
     if (rc) return rc;
     double best = 0.0;
     for (int rep = 0; rep < 6; ++rep) {
         MRF_CUDA(cudaEventRecord(h->ev0, h->stream));
-        fma_peak_kernel<T><<<blocks, threads, 0, h->stream>>>((T*)h->stage[0], iters, T(0.999), T(1e-3));
+        fma_peak_kernel<T><<<blocks, threads, 0, h->stream>>>(out, iters, T(0.999), T(1e-3));
         MRF_CUDA(cudaGetLastError());
         MRF_CUDA(cudaEventRecord(h->ev1, h->stream));
         MRF_CUDA(cudaStreamSynchronize(h->stream));
@@ -2912,7 +2796,7 @@ template <typename T> static int fma_peak(mrf_handle_t h, double* tflops) {
     if (sizeof(T) == 4) { // the FP32 pipe peak is reached with packed FFMA2 (scalar FFMA is issue-limited to ~93 %)
         for (int rep = 0; rep < 6; ++rep) {
             MRF_CUDA(cudaEventRecord(h->ev0, h->stream));
-            fma2_peak_kernel<<<blocks, threads, 0, h->stream>>>((float*)h->stage[0], iters, 0.999f, 1e-3f);
+            fma2_peak_kernel<<<blocks, threads, 0, h->stream>>>((float*)out, iters, 0.999f, 1e-3f);
             MRF_CUDA(cudaGetLastError());
             MRF_CUDA(cudaEventRecord(h->ev1, h->stream));
             MRF_CUDA(cudaStreamSynchronize(h->stream));
