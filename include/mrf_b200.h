@@ -465,6 +465,31 @@ int mrf_point_episode_run_dev_f32(mrf_handle_t h, const MrfPointEpisode* ep, int
  * above.  Default 512; 0 disables the cooperative kernel. */
 int mrf_set_coop_max_batch(mrf_handle_t h, int64_t max_batch);
 
+/* Self-collision pairs (fabrics set_components(..., self_collision_pairs)).  A pair (a, b) of links of one robot is a
+ * 1-D leaf on x = |p_a - p_b| / rho - 1 (p = link origin, rho = r_a + r_b given per pair):
+ *   Finsler energy L = k_f s_f xdot^2 / x^p_f,  geometry h = k_g s_g xdot^2 / x^p_g,
+ *   s = -0.5 (sign(xdot) - 1) where gate = 1, else 1.
+ * Links are 1..8 (panda_linkN) and 9 (panda_hand, the origin of link 8).  Pairs whose two points coincide identically
+ * ((a, a), (5, 6), (8, 9), both in {1, 2}) are rejected: their leaf is 0/0.  Link 1/2 is the constant link1 origin.
+ * The leaves act in every planner of the handle (the grasp planner with has_collision_links = 0 included).
+ * Defaults (mrf_self_collision_default): k_g = -0.5, p_g = 1, gate_g = 1, k_f = 0.1, p_f = 2, gate_f = 0.
+ * Entries that cannot evaluate the leaves return MRF_EUNSUPPORTED while pairs are set: mrf_rollout_risk_dev_*,
+ * mrf_rfcv_post_dev_f32 with risk != NULL, mrf_rollout_host_submit*, mrf_rfcv_host_submit_f32.  Rollouts with pairs
+ * take the generic throughput kernel at every batch size (no cooperative or uniform 3-robot kernel). */
+#define MRF_MAX_SELF_PAIRS 8
+typedef struct MrfSelfCollision {
+    int32_t struct_size;                                    /* sizeof(MrfSelfCollision) */
+    int32_t n_pairs[MRF_MAX_ROBOTS];                        /* 0..MRF_MAX_SELF_PAIRS per robot */
+    int32_t links[MRF_MAX_ROBOTS][MRF_MAX_SELF_PAIRS][2];   /* 1..9 */
+    double rho[MRF_MAX_ROBOTS][MRF_MAX_SELF_PAIRS];         /* > 0 */
+    double k_geometry, k_finsler;
+    int32_t p_geometry, p_finsler;                          /* 1..8 */
+    int32_t gate_geometry, gate_finsler;                    /* 0 / 1 */
+} MrfSelfCollision;
+int mrf_self_collision_default(MrfSelfCollision* sc);      /* zero pairs, the default leaf */
+/* sc == NULL or every n_pairs 0 clears the pairs (the handle then behaves as one that never had any). */
+int mrf_set_self_collision(mrf_handle_t h, const MrfSelfCollision* sc);
+
 /* Number of kernels this library has launched through handle h since creation (for bench accounting). */
 int64_t mrf_launch_count(mrf_handle_t h);
 /* Device time in ms of the last *_host_* call's kernel(s) (CUDA events on the handle's stream). */

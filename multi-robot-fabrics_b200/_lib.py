@@ -68,6 +68,18 @@ class MrfPointEpisode(C.Structure):
     ]
 
 
+MAX_SELF_PAIRS = 8  # MRF_MAX_SELF_PAIRS
+
+
+class MrfSelfCollision(C.Structure):
+    """include/mrf_b200.h: self-collision pairs and their leaf (mrf_set_self_collision)."""
+    _fields_ = [
+        ("struct_size", C.c_int32), ("n_pairs", C.c_int32 * 4), ("links", ((C.c_int32 * 2) * MAX_SELF_PAIRS) * 4),
+        ("rho", (C.c_double * MAX_SELF_PAIRS) * 4), ("k_geometry", C.c_double), ("k_finsler", C.c_double),
+        ("p_geometry", C.c_int32), ("p_finsler", C.c_int32), ("gate_geometry", C.c_int32), ("gate_finsler", C.c_int32),
+    ]
+
+
 _lib = None
 _F = {"f32": (C.c_float, np.float32), "f64": (C.c_double, np.float64)}
 
@@ -87,6 +99,7 @@ EXPORTS = [
     "mrf_rfcv_post_dev_f32", "mrf_rfcv_post_dev_f64", "mrf_rollout_risk_dev_f32", "mrf_rollout_risk_dev_f64",
     "mrf_set_guard", "mrf_guard_stats", "mrf_rollout_static_dev_f32", "mrf_rollout_static_dev_f64",
     "mrf_rfcv_host_submit_f32", "mrf_point_episode_run_dev_f64", "mrf_point_episode_run_dev_f32",
+    "mrf_self_collision_default", "mrf_set_self_collision",
 ]
 
 
@@ -144,6 +157,8 @@ def lib():
     L.mrf_point_episode_run_dev_f64.argtypes = [vp, C.POINTER(MrfPointEpisode), i64, i32, vp]
     L.mrf_point_episode_run_dev_f32.argtypes = [vp, C.POINTER(MrfPointEpisode), i64, i32, vp]
     L.mrf_fma_peak.argtypes = [vp, i32, C.POINTER(C.c_double)]
+    L.mrf_self_collision_default.argtypes = [C.POINTER(MrfSelfCollision)]
+    L.mrf_set_self_collision.argtypes = [vp, C.POINTER(MrfSelfCollision)]
     _lib = L
     return L
 

@@ -11,7 +11,7 @@ import ctypes as C
 import numpy as np
 
 from . import _lib
-from ._lib import DOF, NLINKS, OBST, REC, Handle, MrfError, check, default_config, hptr, lib
+from ._lib import DOF, MAX_SELF_PAIRS, NLINKS, OBST, REC, Handle, MrfError, MrfSelfCollision, check, default_config, hptr, lib
 
 _NP = {"f64": np.float64, "f32": np.float32}
 
@@ -285,6 +285,36 @@ class Fabrics:
         b = None if bands is None else (C.c_double * 6)(*[float(v) for v in bands])
         e = None if risk_edges is None else (C.c_double * 2)(*[float(v) for v in risk_edges])
         check(lib().mrf_set_guard(self.handle.ptr, b, e, band_dist, cap), "mrf_set_guard")
+
+    def set_self_collision(self, pairs=None, rho=None, leaf=None):
+        """Self-collision leaves (fabrics self_collision_pairs), see mrf_set_self_collision.
+
+        pairs: per robot a list of (a, b) link numbers, 1..8 = panda_linkN, 9 = panda_hand; rho: per robot the list of
+        r_a + r_b of each pair; leaf: dict overriding k_geometry, p_geometry, gate_geometry, k_finsler, p_finsler,
+        gate_finsler (defaults: fabrics' self_collision_geometry / self_collision_finsler, DESIGN.md A13).
+        None or no pairs at all clears them."""
+        sc = MrfSelfCollision()
+        check(lib().mrf_self_collision_default(C.byref(sc)), "mrf_self_collision_default")
+        for k, v in (leaf or {}).items():
+            if k not in ("k_geometry", "p_geometry", "gate_geometry", "k_finsler", "p_finsler", "gate_finsler"):
+                raise MrfError(f"unknown self-collision leaf field {k}")
+            setattr(sc, k, v)
+        pairs = pairs or []
+        if len(pairs) > self.n_robots:
+            raise MrfError(f"pairs: one list per robot, the handle has {self.n_robots}")
+        if any(pairs) and (rho is None or len(rho) != len(pairs)):
+            raise MrfError("rho: one list of pair radii per robot of `pairs`")
+        for r, pr in enumerate(pairs):
+            rr = rho[r]
+            if len(pr) != len(rr):
+                raise MrfError(f"robot {r}: {len(pr)} pairs but {len(rr)} radii")
+            if len(pr) > MAX_SELF_PAIRS:
+                raise MrfError(f"robot {r}: at most {MAX_SELF_PAIRS} self-collision pairs")
+            sc.n_pairs[r] = len(pr)
+            for k, ((a, b), rk) in enumerate(zip(pr, rr)):
+                sc.links[r][k][0], sc.links[r][k][1] = int(a), int(b)
+                sc.rho[r][k] = float(rk)
+        check(lib().mrf_set_self_collision(self.handle.ptr, C.byref(sc)), "mrf_set_self_collision")
 
     def guard_stats(self):
         """(re-rolled so far, overflow so far, listed by the last call); synchronise first."""

@@ -348,9 +348,9 @@ template <typename T> struct RollExtra {
     DlPost dl;
 };
 
-template <typename T, int R, bool UNIFORM, bool AOS, bool STRIDE = false>
+template <typename T, int R, bool UNIFORM, bool AOS, bool STRIDE = false, bool SELF = false>
 __global__ void __launch_bounds__(kTile* R, (R == 3 && sizeof(T) == 4) ? MRF_ROLLOUT_MINBLOCKS : MRF_ROLLOUT_MINBLOCKS_F64)
-    rollout_kernel(const __grid_constant__ DevCfg<T> cfg, const T* __restrict__ rec, int N, T* __restrict__ avg_vel,
+    rollout_kernel(const __grid_constant__ CfgOf<T, SELF> cfg, const T* __restrict__ rec, int N, T* __restrict__ avg_vel,
                    T* __restrict__ x_ee, T* __restrict__ goal_est, T* __restrict__ qN, T* __restrict__ qdN, long long B,
                    unsigned* __restrict__ sync, unsigned window, int n_var, const T* __restrict__ rec_tail,
                    T* __restrict__ risk, const __grid_constant__ RollExtra<T> ex) {
@@ -507,7 +507,8 @@ __global__ void __launch_bounds__(kTile* R, (R == 3 && sizeof(T) == 4) ? MRF_ROL
             fabric_action(cfg, r, q, qd, ch, kin, prm, NT, tid, src, act, &stiff, kPair ? &pl : nullptr);
         } else {
             SmemSrc<T> src{cfg, kin, NT, lane, r, vref, aref, st_sph, AOS ? 0 : n_static, tid};
-            fabric_action(cfg, r, q, qd, ch, kin, prm, NT, tid, src, act, &stiff);
+            if constexpr (SELF) fabric_action<T>(cfg, r, q, qd, ch, kin, prm, NT, tid, src, act, &stiff, nullptr, cfg.self);
+            else fabric_action(cfg, r, q, qd, ch, kin, prm, NT, tid, src, act, &stiff);
         }
         prm[P_RISK * NT + tid] = Mth<T>::max(prm[P_RISK * NT + tid], stiff);
 #pragma unroll
@@ -558,9 +559,9 @@ constexpr int kActThreads = 128;
 #ifndef MRF_ACTION_MINBLOCKS
 #define MRF_ACTION_MINBLOCKS 1
 #endif
-template <typename T, bool CART>
+template <typename T, bool CART, bool SELF = false>
 __global__ void __launch_bounds__(kActThreads, sizeof(T) == 4 ? MRF_ACTION_MINBLOCKS : 1)
-    action_kernel(const __grid_constant__ DevCfg<T> cfg, int robot_first, int n_rob, const T* __restrict__ rec, int S,
+    action_kernel(const __grid_constant__ CfgOf<T, SELF> cfg, int robot_first, int n_rob, const T* __restrict__ rec, int S,
                   const T* __restrict__ obst, int N, T* __restrict__ out, T* __restrict__ qN, T* __restrict__ qdN,
                   long long B, const int32_t* __restrict__ sm_state) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -591,7 +592,8 @@ __global__ void __launch_bounds__(kActThreads, sizeof(T) == 4 ? MRF_ACTION_MINBL
     if (!CART) {
         T act[kDof];
         chain_forward(cfg, r, q, qd, ch, kin, NT, tid);
-        fabric_action(cfg, r, q, qd, ch, kin, prm, NT, tid, src, act);
+        if constexpr (SELF) fabric_action<T>(cfg, r, q, qd, ch, kin, prm, NT, tid, src, act, nullptr, nullptr, cfg.self);
+        else fabric_action(cfg, r, q, qd, ch, kin, prm, NT, tid, src, act);
         if (live) {
 #pragma unroll
             for (int i = 0; i < kDof; ++i) out[(long long)i * stride + idx] = act[i];
@@ -605,7 +607,8 @@ __global__ void __launch_bounds__(kActThreads, sizeof(T) == 4 ? MRF_ACTION_MINBL
             T act[kDof];
             src.tk = T(k) * cfg.dt;
             chain_forward(cfg, r, q, qd, ch, kin, NT, tid);
-            fabric_action(cfg, r, q, qd, ch, kin, prm, NT, tid, src, act);
+            if constexpr (SELF) fabric_action<T>(cfg, r, q, qd, ch, kin, prm, NT, tid, src, act, nullptr, nullptr, cfg.self);
+            else fabric_action(cfg, r, q, qd, ch, kin, prm, NT, tid, src, act);
 #pragma unroll
             for (int i = 0; i < kDof; ++i) {
                 if (cfg.mode == 1) { // 'vel': the action is the new velocity (system_step, forward_planner_Cartesian.py:85-87)
@@ -1139,6 +1142,11 @@ struct MrfHandle_ {
     int device;
     DevCfg<float> c32;
     DevCfg<double> c64;
+    // self-collision pairs (mrf_set_self_collision): self_on selects the kernels instantiated with the pair loop, which take
+    // the configuration with the pair table appended
+    int self_on;
+    DevCfgSelf<float> x32;
+    DevCfgSelf<double> x64;
     cudaStream_t stream, s_copy, s_chunk[8];
     cudaEvent_t ev0, ev1, ev_up[8], ev_free, ev_chunk[8];
     // device scratch of the synchronous host entries (scratch_reset / scratch_take): blocks, the last one being filled
@@ -1350,6 +1358,82 @@ extern "C" int mrf_destroy(mrf_handle_t h) {
     return MRF_OK;
 }
 
+extern "C" int mrf_self_collision_default(MrfSelfCollision* sc) {
+    if (!sc) return fail(MRF_EINVAL, "mrf_self_collision_default: null argument");
+    memset(sc, 0, sizeof(*sc));
+    sc->struct_size = (int32_t)sizeof(MrfSelfCollision);
+    // fabrics 0.9.5 self_collision_geometry / self_collision_finsler as recalled (DESIGN.md assumption A13):
+    // "-0.5 / (x ** 1) * (-0.5 * (ca.sign(xdot) - 1)) * xdot ** 2", "0.1/(x**2) * xdot**2"
+    sc->k_geometry = -0.5;
+    sc->p_geometry = 1;
+    sc->gate_geometry = 1;
+    sc->k_finsler = 0.1;
+    sc->p_finsler = 2;
+    sc->gate_finsler = 0;
+    return MRF_OK;
+}
+
+template <typename T> static void fill_self(const MrfSelfCollision& sc, const DevCfg<T>& base, DevCfgSelf<T>& d) {
+    static_cast<DevCfg<T>&>(d) = base;
+    memset(&d.self, 0, sizeof(d.self));
+    // point-table slot and Jacobian column count of panda_link1..8 and panda_hand (index 0 unused)
+    const int slot[10] = {0, 5, 5, 0, 1, 2, 2, 3, 4, 4}, cols[10] = {0, 0, 0, 2, 3, 4, 4, 6, 6, 6};
+    for (int r = 0; r < MRF_MAX_ROBOTS; ++r) {
+        d.self.n[r] = sc.n_pairs[r];
+        for (int k = 0; k < sc.n_pairs[r]; ++k) {
+            for (int s = 0; s < 2; ++s) {
+                d.self.pt[r][k][s] = slot[sc.links[r][k][s]];
+                d.self.K[r][k][s] = cols[sc.links[r][k][s]];
+            }
+            d.self.rho[r][k] = (T)sc.rho[r][k];
+        }
+    }
+    d.self.kg = (T)sc.k_geometry;
+    d.self.kf = (T)sc.k_finsler;
+    d.self.pg = sc.p_geometry;
+    d.self.pf = sc.p_finsler;
+    d.self.gg = sc.gate_geometry;
+    d.self.gf = sc.gate_finsler;
+}
+
+extern "C" int mrf_set_self_collision(mrf_handle_t h, const MrfSelfCollision* sc) {
+    if (!h) return fail(MRF_EINVAL, "mrf_set_self_collision: null handle");
+    int total = 0;
+    if (sc) {
+        if (sc->struct_size != (int32_t)sizeof(MrfSelfCollision))
+            return fail(MRF_EINVAL, "mrf_set_self_collision: struct_size mismatch");
+        for (int r = 0; r < MRF_MAX_ROBOTS; ++r) {
+            const int n = sc->n_pairs[r];
+            if (n < 0 || n > MRF_MAX_SELF_PAIRS) return fail(MRF_EINVAL, "mrf_set_self_collision: n_pairs out of 0..MRF_MAX_SELF_PAIRS");
+            if (n > 0 && r >= h->cfg.n_robots) return fail(MRF_EINVAL, "mrf_set_self_collision: pairs for a robot the handle does not have");
+            for (int k = 0; k < n; ++k) {
+                int a = sc->links[r][k][0], b = sc->links[r][k][1];
+                if (a < 1 || a > 9 || b < 1 || b > 9) return fail(MRF_EINVAL, "mrf_set_self_collision: link out of 1..9");
+                if (a > b) { const int t = a; a = b; b = t; }
+                // the two points coincide identically (same link, link5/6, link8/hand, link1/2): the leaf is 0/0
+                if (a == b || (a == 5 && b == 6) || (a == 8 && b == 9) || b <= 2)
+                    return fail(MRF_EINVAL, "mrf_set_self_collision: the pair's two points coincide");
+                if (!(sc->rho[r][k] > 0.0)) return fail(MRF_EINVAL, "mrf_set_self_collision: rho must be positive");
+            }
+            total += n;
+        }
+        if (sc->p_geometry < 1 || sc->p_geometry > 8 || sc->p_finsler < 1 || sc->p_finsler > 8)
+            return fail(MRF_EINVAL, "mrf_set_self_collision: exponents must be integers in 1..8");
+        if ((sc->gate_geometry != 0 && sc->gate_geometry != 1) || (sc->gate_finsler != 0 && sc->gate_finsler != 1))
+            return fail(MRF_EINVAL, "mrf_set_self_collision: gates must be 0 or 1");
+        if (!std::isfinite(sc->k_geometry) || !std::isfinite(sc->k_finsler))
+            return fail(MRF_EINVAL, "mrf_set_self_collision: coefficients must be finite");
+    }
+    if (total == 0) {
+        h->self_on = 0;
+        return MRF_OK;
+    }
+    fill_self(*sc, h->c32, h->x32);
+    fill_self(*sc, h->c64, h->x64);
+    h->self_on = 1;
+    return MRF_OK;
+}
+
 extern "C" int mrf_set_coop_max_batch(mrf_handle_t h, int64_t max_batch) {
     if (!h || max_batch < 0) return fail(MRF_EINVAL, "mrf_set_coop_max_batch: bad argument");
     h->coop_max_batch = max_batch;
@@ -1361,6 +1445,9 @@ extern "C" double mrf_last_kernel_ms(mrf_handle_t h) { return h ? h->last_ms : 0
 template <typename T> static const DevCfg<T>& devcfg(mrf_handle_t h);
 template <> const DevCfg<float>& devcfg<float>(mrf_handle_t h) { return h->c32; }
 template <> const DevCfg<double>& devcfg<double>(mrf_handle_t h) { return h->c64; }
+template <typename T> static const DevCfgSelf<T>& devcfg_self(mrf_handle_t h);
+template <> const DevCfgSelf<float>& devcfg_self<float>(mrf_handle_t h) { return h->x32; }
+template <> const DevCfgSelf<double>& devcfg_self<double>(mrf_handle_t h) { return h->x64; }
 
 template <typename K> static int set_smem(K kernel, size_t bytes) {
     if (bytes > 48 * 1024) MRF_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
@@ -1392,6 +1479,35 @@ static int rollout_dev(mrf_handle_t h, const T* rec, int N, T* avg_vel, T* x_ee,
     if (aos && (qN || qdN)) return fail(MRF_EINVAL, "mrf_rollout: record-order input has no trajectory output");
     if (n_static < 0 || n_static > MRF_MAX_STATIC || (n_static > 0 && (!stat || aos || n_live)))
         return fail(MRF_EINVAL, "mrf_rollout: bad static-obstacle arguments");
+    if (h->self_on) {
+        // self-collision pairs: only the generic throughput kernel evaluates them (the cooperative and the uniform 3-robot
+        // kernels have their own action code), so every batch size takes it
+        if (risk || n_live) return fail(MRF_EUNSUPPORTED, "mrf_rollout_risk / FP64 guard re-roll: not available with self-collision pairs");
+        if (aos) return fail(MRF_EUNSUPPORTED, "mrf_rollout (host records read in place): not available with self-collision pairs");
+        const size_t smem_s = sizeof(T) * (size_t)(kKinRows<T> + P_N + 4 * n_static) * NT;
+        const long long grid_s = (B + kTile - 1) / kTile;
+        int rc_s = MRF_OK;
+#define MRF_LAUNCH_ROLLOUT_SELF(RR)                                                                                  \
+    case RR:                                                                                                         \
+        rc_s = set_smem(rollout_kernel<T, RR, false, false, false, true>, smem_s);                                   \
+        same_carveout(rollout_kernel<T, RR, false, false, false, true>);                                             \
+        if (rc_s) return rc_s;                                                                                       \
+        rollout_kernel<T, RR, false, false, false, true><<<(unsigned)grid_s, NT, smem_s, (cudaStream_t)stream>>>(    \
+            devcfg_self<T>(h), rec, N, avg_vel, x_ee, goal_est, qN, qdN, (long long)B, h->d_sync + 2 * sync_slot,   \
+            (unsigned)h->zc_window, n_var, rec_tail, nullptr, ex);                                                   \
+        break;
+        switch (R) {
+            MRF_LAUNCH_ROLLOUT_SELF(1)
+            MRF_LAUNCH_ROLLOUT_SELF(2)
+            MRF_LAUNCH_ROLLOUT_SELF(3)
+            MRF_LAUNCH_ROLLOUT_SELF(4)
+            default: return fail(MRF_EINVAL, "mrf_rollout: n_robots out of range");
+        }
+#undef MRF_LAUNCH_ROLLOUT_SELF
+        MRF_CUDA(cudaGetLastError());
+        h->launches += 1;
+        return MRF_OK;
+    }
     if (!aos && R >= 2 && B <= h->coop_max_batch && !risk && !n_live && n_static == 0) {
         // few scenarios: latency matters, not throughput -> one CTA per scenario, one warp per robot (mrf_coop.cuh)
         switch (R) {
@@ -1468,10 +1584,19 @@ static int action_dev(mrf_handle_t h, int robot_first, int n_rob, const T* rec, 
     static const int env_thr = getenv("MRF_ACTION_THREADS_F64") ? atoi(getenv("MRF_ACTION_THREADS_F64")) : 32;
     const int threads = sizeof(T) == 8 ? env_thr : kActThreads;
     const size_t smem = sizeof(T) * (size_t)(kKinRows<T> + P_N + kObstRing * MRF_OBST) * threads;
-    int rc = set_smem(action_kernel<T, CART>, smem);
-    if (rc) return rc;
     const long long total = (long long)n_rob * B;
     const long long grid = (total + threads - 1) / threads;
+    if (h->self_on) { // self-collision pairs: the same kernel with the pair loop (mrf_set_self_collision)
+        int rc = set_smem(action_kernel<T, CART, true>, smem);
+        if (rc) return rc;
+        action_kernel<T, CART, true><<<(unsigned)grid, threads, smem, (cudaStream_t)stream>>>(
+            devcfg_self<T>(h), robot_first, n_rob, rec, S, obst, N, out, qN, qdN, (long long)B, sm_state);
+        MRF_CUDA(cudaGetLastError());
+        h->launches += 1;
+        return MRF_OK;
+    }
+    int rc = set_smem(action_kernel<T, CART>, smem);
+    if (rc) return rc;
     action_kernel<T, CART><<<(unsigned)grid, threads, smem, (cudaStream_t)stream>>>(
         devcfg<T>(h), robot_first, n_rob, rec, S, obst, N, out, qN, qdN, (long long)B, sm_state);
     MRF_CUDA(cudaGetLastError());
@@ -1658,6 +1783,7 @@ static int rfcv_post_dev(mrf_handle_t h, const T* rec, int N, const T* x_ee, T* 
     const bool est = h->cfg.estimate_goal != 0 && goal_est != nullptr;
     const DlOverride ov{nullptr, nullptr, nullptr, nullptr, 0, nullptr};
     if (sizeof(T) == 4 && risk != nullptr) {
+        if (h->self_on) return fail(MRF_EUNSUPPORTED, "mrf_rfcv_post_dev_f32 with risk: the FP64 guard re-roll has no self-collision pairs");
         if (R < 2 || R > 4) return fail(MRF_EINVAL, "mrf_rfcv_post: n_robots must be 2..4");
         MRF_CUDA(cudaSetDevice(h->device));
         cudaStream_t st = (cudaStream_t)stream;
@@ -1976,7 +2102,9 @@ static int rollout_host(mrf_handle_t h, const T* rec, int N, T* avg_vel, T* x_ee
     int rc = scratch_reset(h);
     if (rc) return rc;
     if (!qN && !qdN && B >= 8192) {
-        if (h->zero_copy)
+        // the in-place path reads host records with the rollout kernel's record mode, which has no self-collision variant:
+        // with pairs the records are staged like the other large batches
+        if (h->zero_copy && !h->self_on)
             if (const T* view = (const T*)pinned_view(rec)) return rollout_host_zerocopy<T>(h, view, N, avg_vel, x_ee, goal_est, B);
         return rollout_host_pipelined<T>(h, rec, N, avg_vel, x_ee, goal_est, B);
     }
@@ -2020,6 +2148,7 @@ static int rollout_host_submit(mrf_handle_t h, const T* rec, int N, T* avg_vel, 
                                const T* shared = nullptr) {
     if (!h || !rec) return fail(MRF_EINVAL, "mrf_rollout_host_submit: null argument");
     if (B <= 0 || N <= 0) return fail(MRF_EINVAL, "mrf_rollout_host_submit: B and N must be positive");
+    if (h->self_on) return fail(MRF_EUNSUPPORTED, "mrf_rollout_host_submit: not available with self-collision pairs");
     MRF_CUDA(cudaSetDevice(h->device));
     const T* view = (const T*)pinned_view(rec);
     T* outs[3] = {avg_vel, x_ee, goal_est};
@@ -2104,6 +2233,7 @@ extern "C" int mrf_rfcv_host_submit_f32(mrf_handle_t h, const float* rec, const 
                                         float* result, float* goals_out, int64_t B) {
     if (!h || !rec || !result) return fail(MRF_EINVAL, "mrf_rfcv_host_submit: null argument");
     if (B <= 0 || N <= 0) return fail(MRF_EINVAL, "mrf_rfcv_host_submit: B and N must be positive");
+    if (h->self_on) return fail(MRF_EUNSUPPORTED, "mrf_rfcv_host_submit_f32: not available with self-collision pairs");
     const int R = h->cfg.n_robots;
     if (R < 2) return fail(MRF_EINVAL, "mrf_rfcv_host_submit: the deadlock heuristic needs n_robots >= 2");
     MRF_CUDA(cudaSetDevice(h->device));

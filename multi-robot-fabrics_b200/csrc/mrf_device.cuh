@@ -277,6 +277,30 @@ template <typename T> struct DevCfg {
     T ent_w[MRF_MAX_ROBOTS][kMaxEnt];
 };
 
+// Self-collision pairs of each robot (mrf_set_self_collision), resolved to point-table slots: pt = slot of each link's
+// point (link1/2 -> 5, 3 -> 0, 4 -> 1, 5/6 -> 2, 7 -> 3, 8/hand -> 4), K = Jacobian columns of that point (0 for the
+// constant link1 origin).  Only the kernels instantiated with self-collision take it (DevCfgSelf), so the parameter
+// block of every other kernel is unchanged.
+constexpr int kMaxSelfPairs = MRF_MAX_SELF_PAIRS;
+template <typename T> struct SelfTab {
+    int n[MRF_MAX_ROBOTS];
+    int pt[MRF_MAX_ROBOTS][kMaxSelfPairs][2];
+    int K[MRF_MAX_ROBOTS][kMaxSelfPairs][2];
+    T rho[MRF_MAX_ROBOTS][kMaxSelfPairs];
+    T kg, kf;            // geometry / Finsler coefficients
+    int pg, pf;          // exponents of 1/x
+    int gg, gf;          // sign gates
+};
+template <typename T> struct DevCfgSelf : DevCfg<T> {
+    SelfTab<T> self;
+};
+struct NoSelf {};
+template <typename S> constexpr bool kIsSelf = true;
+template <> constexpr bool kIsSelf<NoSelf> = false;
+template <typename T, bool SELF> struct CfgSel { using type = DevCfg<T>; };
+template <typename T> struct CfgSel<T, true> { using type = DevCfgSelf<T>; };
+template <typename T, bool SELF> using CfgOf = typename CfgSel<T, SELF>::type;
+
 // per-thread state that persists over the horizon (registers)
 template <typename T> struct Chain {
     V3<T> z[6]; // world axes of joints 1..6 (joint 7 moves no collision point)
@@ -963,10 +987,10 @@ template <typename T> MRF_HD void attractor_scalars(T n, T w, T& dpsi, T& m2) {
 // spheres: f(xo, vo, co, radius, weight) with velocity src.vref * vo and acceleration src.aref * co.  q, qd in registers; own kinematics in kin[..tid]; parameters in
 // prm[k*NT + tid].  Writes act[7] (velocity in 'vel' mode, acceleration in 'acc' mode).
 // ------------------------------------------------------------------------------------------------
-template <typename T, typename Src>
+template <typename T, typename Src, typename Self = NoSelf>
 MRF_HD void fabric_action(const DevCfg<T>& cfg, int r, const T* q, const T* qd, const Chain<T>& ch, const T* kin,
                           const T* prm, int NT, int tid, const Src& src, T* act, T* stiff = nullptr,
-                          const PairLeaves<T>* pair = nullptr) {
+                          const PairLeaves<T>* pair = nullptr, const Self& self = Self{}) {
     const T sigma = cfg.sigma;
     // shared robot-robot leaves (pair_leaves_eval has run for this step): the sphere leaves come from the slots
     const bool pair_on = kPairLeaves && Src::kUniformRadius && pair != nullptr && pair->on;
@@ -1237,6 +1261,59 @@ MRF_HD void fabric_action(const DevCfg<T>& cfg, int r, const T* q, const T* qd, 
     }
 
     if (stiff != nullptr) *stiff = stiff_sum;
+
+    // ---- self-collision leaves (every planner of the handle, grasp planner included): the sphere leaf's closed form on
+    //      the relative point d = p_a - p_b, w = v_a - v_b, c = c_a - c_b with columns J_a - J_b, one rank-1 update each.
+    //      M = 2 k_f s_f / x^p_f, f = M h with h = k_g s_g xdot^2 / x^p_g, f_e = -(p_f / 2) M xdot^2 / x ----
+    if constexpr (kIsSelf<Self>) {
+#pragma unroll 1
+        for (int k = 0; k < self.n[r]; ++k) {
+            const int ea = self.pt[r][k][0], eb = self.pt[r][k][1], Ka = self.K[r][k][0], Kb = self.K[r][k][1];
+            const V3<T> pa = kin_load(kin, NT, tid, ea, 0), pb = kin_load(kin, NT, tid, eb, 0);
+            const V3<T> d = pa - pb;
+            const V3<T> w = kin_load(kin, NT, tid, ea, 3) - kin_load(kin, NT, tid, eb, 3);
+            const V3<T> c = kin_load(kin, NT, tid, ea, 6) - kin_load(kin, NT, tid, eb, 6);
+            const T rho = self.rho[r][k];
+            const T n2 = dot(d, d);
+            const T n = Mth<T>::sqrt(n2);
+            const T gs = Mth<T>::rcp(n * rho);                 // g = d * gs is the gradient of x w.r.t. the relative point
+            const T ix = rho * Mth<T>::rcp(n - rho);            // 1/x
+            const T dw = dot(d, w);
+            const T xd = dw * gs;                               // xdot
+            const T s = xd > T(0) ? T(0) : (xd < T(0) ? T(1) : T(0.5));
+            T ipf = T(1), ipg = T(1);
+            for (int i = 0; i < self.pf; ++i) ipf *= ix;
+            for (int i = 0; i < self.pg; ++i) ipg *= ix;
+            const T Ml = T(2) * self.kf * (self.gf ? s : T(1)) * ipf;
+            const T hh = self.kg * (self.gg ? s : T(1)) * ipg;  // h = hh xdot^2
+            const T Mg = Ml * gs;
+            const T kk = Mg * gs;
+            const T u1 = Ml * (xd * xd);                        // M xdot^2
+            const T fl = u1 * hh;                               // f = M h
+            const T fd = u1 * (hh + T(0.5) * T(self.pf) * ix);  // f - f_e
+            // X = M (J-dot qdot of x without sigma) = Mg (|w|^2 + d.c) - u1 rho / n
+            const T X = Mg * (dot(w, w) + dot(d, c)) - u1 * rho * Mth<T>::rcp(n);
+            const T fq = sigma * X + fl;
+            num += xd * ((sigma - T(1)) * X + fd);
+            T u[6];
+#pragma unroll
+            for (int j = 0; j < 6; ++j) {
+                const V3<T> z = axis_of(ch, kin, NT, tid, j), o = org(j);
+                T uj = T(0);
+                if (j < Ka) uj += dot(d, cross(z, pa - o));
+                if (j < Kb) uj -= dot(d, cross(z, pb - o));
+                u[j] = uj;
+            }
+            const T gf = gs * fq;
+#pragma unroll
+            for (int j = 0; j < 6; ++j) {
+                G.f[j] += u[j] * gf;
+                const T ku = kk * u[j];
+#pragma unroll
+                for (int i = 0; i <= j; ++i) G.M[i][j] -= u[i] * ku;
+            }
+        }
+    }
 
     // ---- q^T M_g q ----
     T qMq = G.m7 * qd[6] * qd[6];

@@ -46,7 +46,7 @@ class BatchedEpisodes:
     def __init__(self, rec: np.ndarray, n_horizon: int = 10, rollout_fabrics: bool = True, resolve_deadlocks: bool = True,
                  estimate_goal: bool = False, static_or_dyn: int = 1, n_obst_per_link: int = 1, device: int = 0,
                  dtype: str = "f32", epsilon: float = 0.05, use_graph: bool = True, blocks=None, start_goal=None,
-                 rollouts: str = "jointspace"):
+                 rollouts: str = "jointspace", self_collision_pairs=None, self_collision_rho=None):
         import torch
         self.torch = torch
         if rollouts not in ROLLOUT_MODELS:
@@ -64,6 +64,15 @@ class BatchedEpisodes:
         est_mode = (2 if self.rollout_model == 1 else 1) if estimate_goal else 0
         self.fab = Fabrics(R, device=device, estimate_goal=est_mode, static_or_dyn=static_or_dyn)
         self.fab.handle.set_coop_max_batch(0 if B > 256 else 1 << 20)
+        # self-collision pairs (Fabrics.set_self_collision): per robot a list of (a, b) link numbers, 9 = panda_hand; rho
+        # defaults to the two links' sphere radii of MrfConfig.r_robots (panda_hand: panda_link8's).  Set here, before the
+        # control step is captured in a CUDA graph: the graph holds the kernels and configuration chosen at capture.
+        if self_collision_pairs is not None and any(self_collision_pairs):
+            rho = self_collision_rho
+            if rho is None:
+                rr = self.fab.cfg.r_robots
+                rho = [[rr[r][min(a, 8) - 1] + rr[r][min(b, 8) - 1] for a, b in pr] for r, pr in enumerate(self_collision_pairs)]
+            self.fab.set_self_collision(self_collision_pairs, rho)
         t = lambda a, dt=None: torch.from_numpy(np.ascontiguousarray(a)).to(self.dev, dtype=dt or self.tdt)
         self.rec = t(to_soa(rec))                                    # (44,R,B): q, qdot rows are the live state
         self.goal0 = self.rec[G0:G0 + 3].permute(1, 0, 2).contiguous().clone()     # (R,3,B) task goals

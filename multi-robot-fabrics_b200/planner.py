@@ -17,10 +17,11 @@ library or a B200 is missing the constructors raise MrfError (no CPU fallback).
 from __future__ import annotations
 
 import math
+import warnings
 
 import numpy as np
 
-from ._lib import ANG, CON, DOF, G0, G1, G2, OBST, Q, QD, RB, REC, W0, W1, W2, MrfError, check, default_config, hptr, lib
+from ._lib import ANG, CON, DOF, G0, G1, G2, MAX_SELF_PAIRS, OBST, Q, QD, RB, REC, W0, W1, W2, MrfError, check, default_config, hptr, lib
 from .api import Fabrics
 
 PANDA_LIMITS = [[-2.8973, 2.8973], [-1.7628, 1.7628], [-2.8973, 2.8973], [-3.0718, -0.0698],
@@ -68,12 +69,46 @@ class PandaGoal:
         self._config = _GoalConfig()
 
 
+def _link_number(name) -> int:
+    """'panda_linkN' -> N, 'panda_hand' -> 9 (the numbering of mrf_set_self_collision)."""
+    if name == "panda_hand":
+        return 9
+    if isinstance(name, str) and name.startswith("panda_link") and name[len("panda_link"):].isdigit():
+        n = int(name[len("panda_link"):])
+        if 1 <= n <= 8:
+            return n
+    raise MrfError(f"self-collision link must be panda_link1..8 or panda_hand, got {name!r}")
+
+
+def self_collision_pair_list(pairs: dict):
+    """fabrics' self_collision_pairs dict {link: [paired links]} -> [(a, b)] link numbers, each unordered pair once.
+    Pairs whose two points coincide identically ((a, a), link5/link6, link8/panda_hand, both in link1/link2) have the leaf
+    0/0; fabrics skips such a pair with a warning and so does this."""
+    out = []
+    for a_name, others in (pairs or {}).items():
+        a = _link_number(a_name)
+        for b_name in others:
+            b = _link_number(b_name)
+            lo, hi = min(a, b), max(a, b)
+            if lo == hi or (lo, hi) in ((5, 6), (8, 9)) or hi <= 2:
+                warnings.warn(f"self-collision pair ({a_name}, {b_name}): the two points coincide, pair skipped")
+                continue
+            if (lo, hi) not in [(min(x), max(x)) for x in out]:
+                out.append((a, b))
+    if len(out) > MAX_SELF_PAIRS:
+        raise MrfError(f"at most {MAX_SELF_PAIRS} self-collision pairs per robot, got {len(out)}")
+    return out
+
+
 class PandaFabricPlanner:
     """compute_action drop-in for the planner built by set_planner_panda."""
 
     def __init__(self, mount: np.ndarray, nr_obst: int, nr_obst_dyn: int, collision_links_nr, i_robot: int = 0,
-                 device: int = 0, limits=PANDA_LIMITS, mode: str = "vel", time_step: float = 0.01, dtype: str = "f64"):
+                 device: int = 0, limits=PANDA_LIMITS, mode: str = "vel", time_step: float = 0.01, dtype: str = "f64",
+                 self_collision_pairs=None):
         self.mount = np.asarray(mount, dtype=np.float64).reshape(4, 4)
+        self.self_pairs = self_collision_pair_list(self_collision_pairs)
+        self.self_rho = None               # rho of each pair as last set on the handle (from compute_action's radii)
         self.i_robot = i_robot
         self.nr_obst, self.nr_obst_dyn = int(nr_obst), int(nr_obst_dyn)
         # Any subset of panda_link1..8 (the reference's signature default is [5]); links with constant fk (panda_link1/2)
@@ -137,8 +172,33 @@ class PandaFabricPlanner:
             obst[o, 9] = float(np.asarray(get("radius_obst_dynamic", "radius_obsts_dynamic")).reshape(-1)[0])
         return rec, obst
 
+    def _self_collision_radii(self, kw: dict):
+        """rho = r_a + r_b of each pair from the radii the reference passes: radius_body_panda_links[str(l)] (or
+        radius_body_panda_link{l}) and radius_body_panda_hand."""
+        links = kw.get("radius_body_panda_links", {})
+
+        def radius(l):
+            if l == 9:
+                if "radius_body_panda_hand" not in kw:
+                    raise MrfError("self-collision pair with panda_hand needs radius_body_panda_hand")
+                return float(np.asarray(kw["radius_body_panda_hand"]).reshape(-1)[0])
+            for v in (kw.get(f"radius_body_panda_link{l}"), links.get(str(l)), links.get(l)):
+                if v is not None:
+                    return float(np.asarray(v).reshape(-1)[0])
+            raise MrfError(f"self-collision pair with panda_link{l} needs radius_body_panda_links['{l}']")
+        return [radius(a) + radius(b) for a, b in self.self_pairs]
+
+    def set_self_collision_radii(self, rho):
+        """Set the pairs' rho on the handle if it changed (one C-ABI call; nothing when the radii are the same)."""
+        rho = [float(r) for r in rho]
+        if rho != self.self_rho:
+            self.fab.set_self_collision([self.self_pairs], [rho])
+            self.self_rho = rho
+
     def compute_action(self, **kwargs) -> np.ndarray:
         rec, obst = self._record_and_obstacles(kwargs)
+        if self.self_pairs:
+            self.set_self_collision_radii(self._self_collision_radii(kwargs))
         act = self.fab.action_host(rec[None, None, :], obst[None, None] if len(obst) else None, dtype=self.dtype)[0, 0]
         act = np.asarray(act, dtype=np.float64)
         if np.linalg.norm(act) < 1e-6:     # fabrics: "avoid too small actions"
@@ -147,12 +207,15 @@ class PandaFabricPlanner:
 
 
 def set_planner_panda(degrees_of_freedom: int = 7, nr_obst=0, nr_obst_dyn=1, collision_links_nr=(5,), urdf_links=None,
-                      mount_param=None, i_robot=0, device: int = 0, dtype: str = "f64"):
-    """Same signature as the reference's set_planner_panda; the URDF constants are compiled into the kernels."""
+                      mount_param=None, i_robot=0, device: int = 0, dtype: str = "f64", *, self_collision_pairs=None):
+    """Same signature as the reference's set_planner_panda; the URDF constants are compiled into the kernels.
+    self_collision_pairs (keyword only): fabrics' dict {"panda_linkN" | "panda_hand": [paired links]}; each pair's rho
+    comes from the radius_body_panda_links / radius_body_panda_hand arguments of compute_action."""
     if degrees_of_freedom != 7:
         raise MrfError("the CUDA path is specialised to the 7-dof Panda chain")
     mount = mount_transform(i_robot, mount_param)
-    return PandaFabricPlanner(mount, nr_obst, nr_obst_dyn, list(collision_links_nr), i_robot, device, dtype=dtype), PandaGoal()
+    return PandaFabricPlanner(mount, nr_obst, nr_obst_dyn, list(collision_links_nr), i_robot, device, dtype=dtype,
+                              self_collision_pairs=self_collision_pairs), PandaGoal()
 
 
 class PointFabricPlanner:
@@ -245,6 +308,22 @@ class ForwardFabricsPlanner:
                              mount=mounts, r_robots=r_full, estimate_goal=int(estimate_goal),
                              collision_links=[list(c) for c in self.collision_links_nrs])
         self.fab = Fabrics(config=cfg, device=device)
+        # self-collision pairs of the planners the rollouts are built from: rho as the planner last set it, otherwise
+        # from this planner's link radii (panda_hand = panda_link8's point and radius)
+        pairs, rhos = [], []
+        for i, p in enumerate(planners):
+            pp = list(getattr(p, "self_pairs", []) or [])
+            rho = getattr(p, "self_rho", None)
+            if pp and rho is None:
+                rad = lambda l, i=i: r_full[i][min(l, 8) - 1]
+                rho = [rad(a) + rad(b) for a, b in pp]
+                if any(r <= 0.0 for r in rho):
+                    raise MrfError(f"robot {i}: a self-collision pair's link has no radius in r_robots; call the planner's "
+                                   "compute_action (or set_self_collision_radii) first")
+            pairs.append(pp)
+            rhos.append(list(rho or []))
+        if any(pairs):
+            self.fab.set_self_collision(pairs, rhos)
 
     def forward_multi_fabrics_symbolic(self):
         """The reference builds the CasADi graph here; the CUDA kernels need no per-configuration compilation."""
