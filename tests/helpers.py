@@ -13,6 +13,16 @@ def rel_ps(got, ref, ok=None):
     return float(e.max() if ok is None else e[ok].max())
 
 
+def err_ps(got, ref):
+    """PER-SCENARIO error with a unit floor: for every scenario (axis 0) max |got - ref| over the remaining axes divided by
+    max(1, max |ref|) -- relative for large values, absolute for small ones.  A non-finite result counts as infinite."""
+    got, ref = np.asarray(got, dtype=np.float64), np.asarray(ref, dtype=np.float64)
+    ax = tuple(range(1, ref.ndim))
+    with np.errstate(invalid="ignore"):
+        e = np.abs(got - ref).max(axis=ax) / np.maximum(1.0, np.abs(ref).max(axis=ax))
+    return np.nan_to_num(e, nan=np.inf)
+
+
 def oracle_rollout(rec, R, N, estimate_goal=0, static_or_dyn=1):
     """Oracle O2 coupled rollout incl. the RF-CV goal estimate; returns qN, qdN, avg, xee, goal_est, ok-mask."""
     ocfg = o2.default_config(R, static_or_dyn=static_or_dyn)
